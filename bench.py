@@ -10,12 +10,15 @@ torchgems.spatial modules (which call libspconv.so through the C ABI).
 
     python bench.py --gpus N --steps K --warmup W            # our arm
     python bench.py --impl reference ...                     # the reference's CPU path (port)
+    python bench.py ... --dump-outputs DIR                   # also save what the last timed step computed
 
-Prints ONE JSON line (see the task contract): metric/value/unit, ms_per_step, e2e, roofline,
-cpu_baseline, clocks, gpu_launches.
+Prints ONE JSON line: metric/value/unit, ms_per_step, e2e, roofline, cpu_baseline, clocks,
+gpu_launches.  Weights and inputs are seeded, so runs with the same arguments compute on identical
+data and two builds can be compared output for output through --dump-outputs.
 """
 import argparse
 import json
+import math
 import os
 import statistics
 import subprocess
@@ -31,6 +34,8 @@ WORKLOADS = {
     "resnet": ("layers_resnet101_sp2.json", "ResNet-v2-101 spatial stage (split_size=2) @ 4096x4096"),
 }
 METRIC = "images/sec (device-timed, max over ranks) AmoebaNet-D 8192^2 hot path (spatial-stage conv/pool fwd+bwd)"
+DUMP_SAMPLE = 65536          # elements sampled per layer output / input gradient by --dump-outputs
+DUMP_MAX_BYTES = 64 << 20
 
 
 _T0 = time.time()
@@ -94,6 +99,12 @@ class ClockSampler:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"]}
         time.sleep(0.15)
         self.proc.terminate()
+        try:                                   # reap it: no sampler may outlive the benchmark
+            self.proc.wait(timeout=10)
+        except subprocess.TimeoutExpired:
+            self.proc.kill()
+            self.proc.wait()
+        self.t.join()
         sm, mx, reasons = [], None, set()
         names = ["hw_slowdown", "hw_thermal_slowdown", "sw_thermal_slowdown", "sw_power_cap"]
         for ts, l in self.lines:
@@ -110,6 +121,19 @@ class ClockSampler:
                     reasons.add(nme)
         return {"sm_mhz": statistics.median(sm) if sm else None, "sm_max_mhz": mx, "reasons": sorted(reasons),
                 "samples": len(sm)}
+
+
+def write_dump(out_dir, arrays):
+    """--dump-outputs: save each tensor of `arrays` (name -> tensor) as out_dir/<name>.npy in float32."""
+    import numpy as np
+
+    host = {k: t.detach().float().cpu().numpy() for k, t in arrays.items()}
+    nbytes = sum(a.nbytes for a in host.values())
+    assert nbytes <= DUMP_MAX_BYTES, "--dump-outputs: %d bytes exceed the %d-byte limit" % (nbytes, DUMP_MAX_BYTES)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in host.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+    _log("wrote %d arrays (%.1f MB) to %s" % (len(host), nbytes / 2**20, out_dir))
 
 
 def conv_bytes_flops(l, tile_h, tile_w, esz):
@@ -397,7 +421,15 @@ def main():
     ap.add_argument("--cudnn-full-size", action="store_true",
                     help="time cuDNN on the whole tile even where a tensor exceeds 2^31-1 elements (adds minutes)")
     ap.add_argument("--no-model-stage", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed (rank 0) as DIR/<name>.npy: "
+                         "the flattened weight gradients, the step's result, and a fixed seeded sample of every distinct "
+                         "layer's output and input gradient (the sampling adds one gather per sampled tensor to the step)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs saves the GPU path's outputs; --impl reference has none")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -437,6 +469,7 @@ def main():
     algo = _lib.SPC_ALGO_DIRECT if args.algo == "direct" else _lib.SPC_ALGO_AUTO
 
     # ---- build one module per distinct layer shape (weights shared by repeats) ------------------
+    torch.manual_seed(0)          # the same weights (and host image) on every rank and in every run
     uniq = {}
     order = []
     for l in d["layers"]:
@@ -490,6 +523,27 @@ def main():
             n *= s
         return buf[:n].view(shape)
 
+    # --dump-outputs: layer outputs and input gradients are tens of GB per step and each is dropped after its layer,
+    # so the step gathers a fixed seeded sample of them, once per distinct layer (repeats compute the same tensors)
+    samples = {}
+    if args.dump_outputs:
+        gen = torch.Generator().manual_seed(4321)
+        for i, key in enumerate(order):
+            u = uniq[key]
+            if order.index(key) != i:
+                continue
+            samples[i] = {}
+            for name, shape in (("output", u["out_shape"]), ("input_grad", None if u["first"] else u["in_shape"])):
+                if shape is not None:
+                    n = math.prod(shape)
+                    idx = torch.randint(n, (min(n, DUMP_SAMPLE),), generator=gen).sort().values.to(dev)
+                    samples[i][name] = (idx, torch.empty(idx.numel(), dtype=dtype, device=dev))
+
+    def take_sample(i, name, t):
+        idx, buf = samples[i][name]
+        with torch.no_grad():
+            torch.index_select(t.reshape(-1), 0, idx, out=buf)
+
     def step_body(from_host_image):
         """One pass of the hot path: every layer fwd + bwd, gradient flatten, allreduce / P."""
         off = 0
@@ -501,7 +555,12 @@ def main():
             if not u["first"]:
                 x.requires_grad_(True)
             y = u["mod"](x)
+            sample = i in samples and not from_host_image
+            if sample:
+                take_sample(i, "output", y)
             y.backward(view(scratch_gy, u["out_shape"]))
+            if sample and "input_grad" in samples[i]:
+                take_sample(i, "input_grad", x.grad)
             x.grad = None
             if u["layer"]["op"] == "conv":
                 w = u["mod"].weight
@@ -515,6 +574,7 @@ def main():
         return last.detach().float().sum().view(1)
 
     graphs = {}
+    last_result = {}
 
     def step(e2e=False):
         """e2e: the step's input image comes from pinned HOST memory and its result goes back to the host."""
@@ -527,6 +587,7 @@ def main():
             res = step_body(e2e)
         if e2e:
             host_out.copy_(res, non_blocking=True)
+        last_result[e2e] = res
 
     def timed(nsteps, e2e):
         if world > 1:
@@ -601,6 +662,13 @@ def main():
     launches = launches_per_step * args.steps
     t_wall1 = time.time()
     clocks = sampler.stop(t_wall0, t_wall1) if sampler else None
+    if args.dump_outputs and rank == 0:
+        # saved before the e2e steps, which overwrite the weight gradients with those of the host image
+        arrays = {"weight_grads": flat_grads, "step_result": last_result[False]}
+        for i, s in samples.items():
+            for name, (_, buf) in s.items():
+                arrays["layer%02d_%s" % (i, name)] = buf
+        write_dump(args.dump_outputs, arrays)
     ms_e2e = timed(args.steps, True)
     _log("timed: %.2f ms/step, e2e %.2f ms/step" % (ms_total / args.steps, ms_e2e / args.steps))
 

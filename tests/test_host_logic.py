@@ -166,3 +166,17 @@ def test_bench_reference_arm_prints_the_contract_line():
     other = subprocess.run(cmd, capture_output=True, text=True, timeout=120, cwd=root,
                            env=dict(env, RANK="1", WORLD_SIZE="2", LOCAL_RANK="1"))
     assert other.returncode == 0 and other.stdout.strip() == "", (other.stdout, other.stderr[-500:])
+
+
+@pytest.mark.parametrize("extra,msg", [(["--steps", "0"], "--steps"),
+                                       (["--impl", "reference", "--dump-outputs", "out"], "--dump-outputs")])
+def test_bench_rejects_bad_arguments(extra, msg, tmp_path):
+    """No timed steps, or a dump the CPU reference arm cannot make, is a usage error before any work starts."""
+    import os
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py")] + extra, capture_output=True, text=True,
+                         timeout=120, cwd=tmp_path, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
+    assert out.returncode == 2 and msg in out.stderr and out.stdout == "", out.stderr[-500:]
+    assert os.listdir(tmp_path) == []
