@@ -31,7 +31,8 @@ from mpi4dl_b200.torchgems.train_spatial_master import train_spatial_model_maste
 
 def main(kind):
     p = parser.get_parser()
-    p.add_argument("--dtype", choices=["fp32", "bf16"], default="fp32")
+    p.add_argument("--dtype", choices=["fp32", "bf16", "tf32"], default="fp32",
+                   help="tf32: fp32 tensors, convolutions on the tensor cores with TF32 operands")
     p.add_argument("--steps", type=int, default=10)
     args = p.parse_args()
     gems_comm.initialize_cuda()
@@ -49,6 +50,10 @@ def main(kind):
         raise NotImplementedError("--local-DP > 1 is not built")
     mb = int(batch_size / parts)
     dtype = torch.bfloat16 if args.dtype == "bf16" else torch.float32
+    if args.dtype == "tf32":
+        from mpi4dl_b200.torchgems.spatial import set_fp32_math
+
+        set_fp32_math("tf32")
 
     comm1 = gems_comm.MPIComm(split_size=split_size, ENABLE_MASTER=False, ENABLE_SPATIAL=True,
                               num_spatial_parts=num_spatial_parts, spatial_size=spatial_size, LOCAL_DP_LP=1)

@@ -85,7 +85,8 @@ def _batches(args, image_size, batch_size, steps):
 
 def main(kind):
     p = parser.get_parser()
-    p.add_argument("--dtype", choices=["fp32", "bf16"], default="fp32")
+    p.add_argument("--dtype", choices=["fp32", "bf16", "tf32"], default="fp32",
+                   help="tf32: fp32 tensors, convolutions on the tensor cores with TF32 operands")
     p.add_argument("--steps", type=int, default=10)
     args = p.parse_args()
     gems_comm.initialize_cuda()
@@ -107,6 +108,10 @@ def main(kind):
     local_rank, split_rank = mpi_comm.rank, mpi_comm.split_rank
     mb = int(batch_size / parts)
     dtype = torch.bfloat16 if args.dtype == "bf16" else torch.float32
+    if args.dtype == "tf32":
+        from mpi4dl_b200.torchgems.spatial import set_fp32_math
+
+        set_fp32_math("tf32")
 
     spatial_kw = dict(input_shape=(mb, 3, image_size, image_size), local_rank=local_rank % P, mp_size=split_size,
                       balance=balance, spatial_size=spatial_size, num_spatial_parts=num_spatial_parts, slice_method=slice_method)

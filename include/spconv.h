@@ -35,7 +35,10 @@ extern "C" {
 enum { SPC_OK = 0, SPC_EINVAL = -1, SPC_ECUDA = -2, SPC_EUNSUPPORTED = -3, SPC_ENOMEM = -4 };
 enum { SPC_F32 = 0, SPC_BF16 = 1 };             /* storage dtype of x / w / y; accumulation is fp32 */
 enum { SPC_POOL_MAX = 0, SPC_POOL_AVG = 1 };
-enum { SPC_ALGO_AUTO = 0, SPC_ALGO_DIRECT = 1, SPC_ALGO_TCGEN05 = 2 };
+/* SPC_ALGO_TF32: like AUTO, but fp32 storage may use the tensor cores with TF32 operands (fp32 accumulate, fp32
+ * output); with bf16 storage it is AUTO.  fp32 shapes the TF32 path does not cover, and the halo boundary rows /
+ * columns of fp32 convolutions, run on the direct kernel in exact fp32.  With AUTO, fp32 is always exact fp32. */
+enum { SPC_ALGO_AUTO = 0, SPC_ALGO_DIRECT = 1, SPC_ALGO_TCGEN05 = 2, SPC_ALGO_TF32 = 3 };
 
 /* Geometry of one spatially-partitioned convolution on one tile.
  * Mirrors conv_spatial.__init__ (spatial.py:26-155): padding is "same"

@@ -8,7 +8,7 @@ LIB_PATH = os.path.join(HERE, "libspconv.so")
 
 SPC_F32, SPC_BF16 = 0, 1
 SPC_POOL_MAX, SPC_POOL_AVG = 0, 1
-SPC_ALGO_AUTO, SPC_ALGO_DIRECT, SPC_ALGO_TCGEN05 = 0, 1, 2
+SPC_ALGO_AUTO, SPC_ALGO_DIRECT, SPC_ALGO_TCGEN05, SPC_ALGO_TF32 = 0, 1, 2, 3
 IPC_HANDLE_BYTES = 64
 
 

@@ -40,10 +40,68 @@ int run_wgrad_tap(const __nv_bfloat16* x, const __nv_bfloat16* dy, float* dw, in
 namespace {
 
 constexpr int TC_THREADS = 192;
-constexpr int BK = 64;                 // channels per pipeline stage (one 128-byte swizzle row of A)
-constexpr int A_BLK_BYTES = 128 * BK * 2;   // one 128-row M block of A per stage: 16 KB
-constexpr int B_BLK_BYTES = BK * 64 * 2;    // one 64-pixel block of B per stage: 8 KB
+constexpr int A_BLK_BYTES = 128 * 128;      // one 128-row M block of A per stage (one 128-byte swizzle row per row): 16 KB
 constexpr int TMEM_COLS = 512;
+
+// Storage types of the tcgen05 GEMMs: bf16 (kind::f16) and fp32 read as TF32 (kind::tf32, opt-in, SPC_ALGO_TF32).
+// One 128-byte swizzle row holds ROW = 64 bf16 or 32 fp32 elements: ROW channels per pipeline stage (K-major A), ROW
+// pixels per B block (MN-major B) and per wgrad chunk.  One MMA reduces 32 bytes of K (16 bf16 / 8 TF32), so a stage is
+// 4 MMA k-steps and every per-stage BYTE count is the same for both types; only the element counts per row change.
+template <typename T> struct Tc;
+template <> struct Tc<__nv_bfloat16> {
+  static constexpr CUtensorMapDataType TMA_TYPE = CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+  // MN-major B operand (fprop / dgrad activations): TMA swizzle and matching UMMA descriptor layout
+  static constexpr CUtensorMapSwizzle B_SWZ = CU_TENSOR_MAP_SWIZZLE_128B;
+  static constexpr uint32_t B_LAYOUT = UMMA_SW128;
+  static constexpr uint32_t B_SBO = 1024;   // 8-row swizzle atoms along K
+  static __host__ __device__ constexpr uint32_t idesc(int M, int N, int a_mn, int b_mn) {
+    return umma_idesc_bf16(M, N, a_mn, b_mn);
+  }
+  static __device__ __forceinline__ void mma(uint32_t d, uint64_t a, uint64_t b, uint32_t id, uint32_t acc) {
+    umma_bf16(d, a, b, id, acc);
+  }
+  static __device__ __forceinline__ float to_float(__nv_bfloat16 v) { return __bfloat162float(v); }
+  static __device__ __forceinline__ __nv_bfloat16 from_float(float v) { return __float2bfloat16(v); }
+  // 8 accumulator columns (+bias) -> one 16-byte chunk of the output row
+  static __device__ __forceinline__ uint4 pack16(const uint32_t* r, float bias) {
+    uint4 v;
+    v.x = pack_bf16x2(__uint_as_float(r[0]) + bias, __uint_as_float(r[1]) + bias);
+    v.y = pack_bf16x2(__uint_as_float(r[2]) + bias, __uint_as_float(r[3]) + bias);
+    v.z = pack_bf16x2(__uint_as_float(r[4]) + bias, __uint_as_float(r[5]) + bias);
+    v.w = pack_bf16x2(__uint_as_float(r[6]) + bias, __uint_as_float(r[7]) + bias);
+    return v;
+  }
+};
+template <> struct Tc<float> {
+  static constexpr CUtensorMapDataType TMA_TYPE = CU_TENSOR_MAP_DATA_TYPE_FLOAT32;
+  // an MN-major TF32 operand is swizzled in 32-byte atoms (a 16-byte chunk holds only 4 fp32 values): four atoms per
+  // 128-byte row, so the pattern repeats every 4 rows and one 8-channel MMA spans two 4-row K groups 512 B apart
+  // (measured on B200, tools/tf32_mma_probe.cu, profiles/r3_tf32_mma_probe.txt).  K-major TF32 uses the plain swizzle.
+  static constexpr CUtensorMapSwizzle B_SWZ = CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B;
+  static constexpr uint32_t B_LAYOUT = UMMA_SW128_ATOM32;
+  static constexpr uint32_t B_SBO = 512;
+  static __host__ __device__ constexpr uint32_t idesc(int M, int N, int a_mn, int b_mn) {
+    return umma_idesc_tf32(M, N, a_mn, b_mn);
+  }
+  static __device__ __forceinline__ void mma(uint32_t d, uint64_t a, uint64_t b, uint32_t id, uint32_t acc) {
+    umma_tf32(d, a, b, id, acc);
+  }
+  static __device__ __forceinline__ float to_float(float v) { return v; }
+  static __device__ __forceinline__ float from_float(float v) { return v; }
+  // 4 accumulator columns (+bias) -> one 16-byte chunk of the output row, no rounding
+  static __device__ __forceinline__ uint4 pack16(const uint32_t* r, float bias) {
+    uint4 v;
+    v.x = __float_as_uint(__uint_as_float(r[0]) + bias);
+    v.y = __float_as_uint(__uint_as_float(r[1]) + bias);
+    v.z = __float_as_uint(__uint_as_float(r[2]) + bias);
+    v.w = __float_as_uint(__uint_as_float(r[3]) + bias);
+    return v;
+  }
+};
+template <typename T> constexpr int ROW = 128 / (int)sizeof(T);         // elements per 128-byte swizzle row
+template <typename T> constexpr int KSTEP = 32 / (int)sizeof(T);        // K per MMA
+template <typename T> constexpr int B_BLK_BYTES = ROW<T> * 128;         // [ROW ch][ROW px] block of B: 8 KB / 4 KB
+constexpr int BK = ROW<__nv_bfloat16>;   // bf16-only paths (stride-2 dgrad repack, boundary GEMM workspace)
 
 // ---- host: TMA descriptor encode (driver entry point fetched through the runtime) -------------
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
@@ -61,9 +119,9 @@ EncodeTiledFn get_encode() {
   return fn;
 }
 
-// bf16 tensor map, rank <= 4; dims/strides innermost first (strides in BYTES for dims 1..).
+// tensor map (bf16 unless told otherwise), rank <= 5; dims/strides innermost first (strides in BYTES for dims 1..).
 int make_tmap_sw(CUtensorMap* m, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
-                 const uint32_t* box, CUtensorMapSwizzle swz) {
+                 const uint32_t* box, CUtensorMapSwizzle swz, CUtensorMapDataType dt = CU_TENSOR_MAP_DATA_TYPE_BFLOAT16) {
   EncodeTiledFn enc = get_encode();
   if (!enc) {
     set_error("cuTensorMapEncodeTiled entry point not available");
@@ -87,7 +145,7 @@ int make_tmap_sw(CUtensorMap* m, const void* base, int rank, const uint64_t* dim
     es[i] = 1;
     if (i > 0) gs[i - 1] = strides_bytes[i];
   }
-  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, (cuuint32_t)rank, const_cast<void*>(base), gd, gs, bx, es,
+  CUresult r = enc(m, dt, (cuuint32_t)rank, const_cast<void*>(base), gd, gs, bx, es,
                    CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
@@ -101,22 +159,23 @@ int make_tmap_sw(CUtensorMap* m, const void* base, int rank, const uint64_t* dim
 }
 
 int make_tmap(CUtensorMap* m, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes,
-              const uint32_t* box) {
-  return make_tmap_sw(m, base, rank, dims, strides_bytes, box, CU_TENSOR_MAP_SWIZZLE_128B);
+              const uint32_t* box, CUtensorMapDataType dt = CU_TENSOR_MAP_DATA_TYPE_BFLOAT16) {
+  return make_tmap_sw(m, base, rank, dims, strides_bytes, box, CU_TENSOR_MAP_SWIZZLE_128B, dt);
 }
 
-// ---- weight repack: Wp[tap][m][c] (bf16, zero padded to [taps][Mpad][Cpad]) -----------------------
+// ---- weight repack: Wp[tap][m][c] (zero padded to [taps][Mpad][Cpad]) ------------------------------
 // element = w[m*sm + c*sc + (flip ? taps-1-tap : tap)]
 //   fprop: m = out channel k, c = in channel:  sm = C*RS, sc = RS, flip = 0     (w is [K][C][R][S])
 //   dgrad: m = c, c = k (transposed) and the filter is rotated by 180 degrees:  sm = RS, sc = C*RS, flip = 1
-__global__ void repack_weights_kernel(const __nv_bfloat16* __restrict__ w, __nv_bfloat16* __restrict__ wp, int M,
+template <typename T>
+__global__ void repack_weights_kernel(const T* __restrict__ w, T* __restrict__ wp, int M,
                                       int Cc, int Mpad, int Cpad, int taps, long long sm, long long sc, int flip) {
   const int total = taps * Mpad * Cpad;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < total; i += gridDim.x * blockDim.x) {
     const int c = i % Cpad;
     const int m = (i / Cpad) % Mpad;
     const int tap = i / (Cpad * Mpad);
-    __nv_bfloat16 v = __float2bfloat16(0.f);
+    T v = Tc<T>::from_float(0.f);
     if (m < M && c < Cc) v = w[(size_t)m * sm + (size_t)c * sc + (flip ? taps - 1 - tap : tap)];
     wp[i] = v;
   }
@@ -124,7 +183,8 @@ __global__ void repack_weights_kernel(const __nv_bfloat16* __restrict__ w, __nv_
 
 // ---- fprop / dgrad kernel -----------------------------------------------------------------------
 constexpr int BN_DEFAULT = 128;               // pixels per tile (two 64-pixel swizzle blocks); 256 in the wide-N variant
-constexpr int OUT_BUF_BYTES = 128 * 128 * 2;  // epilogue staging: one 128-channel block of 128 pixels of a tile
+// epilogue staging: one 128-channel block of 128 pixels of a tile (32 KB bf16, 64 KB fp32)
+template <typename T> constexpr int OUT_BUF_BYTES = 128 * 128 * (int)sizeof(T);
 constexpr int MAX_STAGES = 8;
 
 struct PwParams {
@@ -143,8 +203,8 @@ struct PwParams {
   int shiftN;                  // N when the activations are S column-shifted copies, else 0
   int rowmul;                  // input row = rowmul * output row + tap row offset (2 for stride-2 convs)
   int tgroup;                  // consecutive tiles handled back-to-back by one CTA (DRAM page locality)
-  const __nv_bfloat16* bias;   // [M] or null
-  __nv_bfloat16* y;            // output base [N][M][P] (coalesced-store epilogue)
+  const void* bias;            // [M] or null, storage type
+  void* y;                     // output base [N][M][P] (coalesced-store epilogue)
   int epi_stg;                 // 1: staged tile leaves with per-thread 16-B stores (full 128-B lines), 0: TMA store
   int x5, y5;                  // 1: activations / outputs move as ONE 5-d box per tile whose traversal order is
                                // (8-channel group, 64-pixel block, channel, pixel): the TMA unit touches 8 channel
@@ -157,26 +217,31 @@ struct PwParams {
 
 // EXT = false compiles the round-2 options (5-d boxes, box-row knobs, per-thread-store epilogue) out: the launches that
 // use none of them (every tap-mode launch; the stem is epilogue-bound and ran 16 % slower with the extra branches in
-// its epilogue, A/B on one GPU) get exactly the plain kernel.
-template <int MB, int BN, bool EXT>
+// its epilogue, A/B on one GPU) get exactly the plain kernel.  T = float (TF32 operands) is only built with EXT = false.
+template <typename T, int MB, int BN, bool EXT>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 pw_gemm_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant__ CUtensorMap tmap_x,
                const __grid_constant__ CUtensorMap tmap_x4, const __grid_constant__ CUtensorMap tmap_y,
                const PwParams p) {
-  constexpr int NB = BN / 64;
+  constexpr int BK = ROW<T>;               // channels per pipeline stage (one 128-byte swizzle row of A)
+  constexpr int PXB = ROW<T>;              // pixels per B block (one 128-byte swizzle row of B)
+  constexpr int KS = KSTEP<T>;
+  constexpr int BBLK = B_BLK_BYTES<T>;
+  constexpr int OUTB = OUT_BUF_BYTES<T>;
+  constexpr int NB = BN / PXB;
   constexpr int ACC = (MB <= 2) ? 2 : 1;
   static_assert(ACC * MB * BN <= TMEM_COLS, "TMEM budget");
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
   const int kchunks = (p.Cin + BK - 1) / BK;
-  const int ksteps_total = (p.Cin + 15) / 16;
-  const int iters = p.taps * kchunks;      // K loop: (filter tap, 64-channel chunk)
+  const int ksteps_total = (p.Cin + KS - 1) / KS;
+  const int iters = p.taps * kchunks;      // K loop: (filter tap, BK-channel chunk)
   const int wres_bytes = p.wres ? iters * MB * A_BLK_BYTES : 0;
-  const int stage_bytes = (p.wres ? 0 : MB * A_BLK_BYTES) + NB * B_BLK_BYTES;
+  const int stage_bytes = (p.wres ? 0 : MB * A_BLK_BYTES) + NB * BBLK;
   uint8_t* wres = smem;
   uint8_t* stage0 = smem + wres_bytes;
   uint8_t* outbuf = stage0 + p.stages * stage_bytes;
-  uint64_t* full = reinterpret_cast<uint64_t*>(outbuf + p.out_bufs * OUT_BUF_BYTES);
+  uint64_t* full = reinterpret_cast<uint64_t*>(outbuf + p.out_bufs * OUTB);
   uint64_t* empty = full + MAX_STAGES;
   uint64_t* tfull = empty + MAX_STAGES;
   uint64_t* tempty = tfull + 2;
@@ -242,12 +307,12 @@ pw_gemm_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant
               tma_load_5d(st, &tmap_x, &full[s], 0, 0, p0 >> 6, kc * (BK / 8), n);
             } else if (xbox == BK) {
 #pragma unroll
-              for (int j = 0; j < NB; ++j) tma_load_3d(st + j * B_BLK_BYTES, &tmap_x, &full[s], p0 + j * 64, kc * BK, n);
+              for (int j = 0; j < NB; ++j) tma_load_3d(st + j * BBLK, &tmap_x, &full[s], p0 + j * PXB, kc * BK, n);
             } else {
               for (int cg = 0; cg < BK; cg += xbox)
 #pragma unroll
                 for (int j = 0; j < NB; ++j)
-                  tma_load_3d(st + j * B_BLK_BYTES + cg * 128, &tmap_x, &full[s], p0 + j * 64, kc * BK + cg, n);
+                  tma_load_3d(st + j * BBLK + cg * 128, &tmap_x, &full[s], p0 + j * PXB, kc * BK + cg, n);
             }
           } else {
             // shifted window of this tap; out-of-image rows / columns are zero-filled by TMA (= zero padding)
@@ -255,8 +320,8 @@ pw_gemm_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant
             const int img = n + (tap % p.S) * p.shiftN;   // column shift = which pre-shifted copy
 #pragma unroll
             for (int j = 0; j < NB; ++j) {
-              const int q = p0 + j * 64, hq = q / p.W, wq = q - hq * p.W;
-              tma_load_4d(st + j * B_BLK_BYTES, &tmap_x4, &full[s], wq, hq * p.rowmul + dr, kc * BK, img);
+              const int q = p0 + j * PXB, hq = q / p.W, wq = q - hq * p.W;
+              tma_load_4d(st + j * BBLK, &tmap_x4, &full[s], wq, hq * p.rowmul + dr, kc * BK, img);
             }
           }
           if (++s == p.stages) { s = 0; ph ^= 1; }
@@ -266,7 +331,7 @@ pw_gemm_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant
   } else if (warp == 1) {
     // ================= MMA issuer =================
     if (lane == 0) {
-      constexpr uint32_t IDESC = umma_idesc_bf16(128, BN, /*a_mn=*/0, /*b_mn=*/1);
+      constexpr uint32_t IDESC = Tc<T>::idesc(128, BN, /*a_mn=*/0, /*b_mn=*/1);
       if (p.wres) { mbar_wait(wfull, 0); tc_fence_after(); }
       int s = 0, ph = 0, a = 0, aph = 0;
       for (int it = 0;; ++it) {
@@ -284,15 +349,17 @@ pw_gemm_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant
           const uint32_t sb = p.wres ? st : st + MB * A_BLK_BYTES;
           const int nsteps = min(4, ksteps_total - kc * 4);
           for (int ks = 0; ks < nsteps; ++ks) {
-            // B: MN-major SW128. 16 channels = two 8-row groups (SBO = 1024 B); 64-px blocks at LBO = 8 KB
+            // B: MN-major SW128. KS channels = KS rows of 128 B (K groups at SBO); PXB-px blocks at LBO = BBLK
+            // (bf16: 16 channels = two 8-row groups, 64-px blocks at 8 KB; TF32: 8 channels = two 4-row groups of
+            // 32-byte atoms, 32-px blocks at 4 KB)
             // (5-d box layout [8-ch group][px block][8 ch][128 B]: px blocks at LBO = 1 KB, channel groups at SBO = 2 KB)
             const uint64_t bdesc = x5 ? umma_desc(sb + ks * (NB * 2048), 1024, NB * 1024)
-                                        : umma_desc(sb + ks * 2048, B_BLK_BYTES, 1024);
+                                        : umma_desc(sb + ks * (KS * 128), BBLK, Tc<T>::B_SBO, Tc<T>::B_LAYOUT);
 #pragma unroll
             for (int mb = 0; mb < MB; ++mb) {
-              // A: K-major SW128. 8-row groups at SBO = 1024 B; +32 B per 16-channel k-step
+              // A: K-major SW128. 8-row groups at SBO = 1024 B; +32 B per k-step
               const uint64_t adesc = umma_desc(sa + mb * A_BLK_BYTES + ks * 32, 16, 1024);
-              umma_bf16(tmem_base + (a * MB + mb) * BN, adesc, bdesc, IDESC, (it | ks) ? 1u : 0u);
+              Tc<T>::mma(tmem_base + (a * MB + mb) * BN, adesc, bdesc, IDESC, (it | ks) ? 1u : 0u);
             }
           }
           umma_commit(&empty[s]);
@@ -323,11 +390,11 @@ pw_gemm_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant
         const int k0 = mg * (MB * 128) + mb * 128;
         if (k0 >= p.M) break;                       // block-uniform: nothing valid in this block
         const int k = k0 + row;
-        const float bias = (k < p.M && p.bias) ? __bfloat162float(p.bias[k]) : 0.f;
+        const float bias = (k < p.M && p.bias) ? Tc<T>::to_float(static_cast<const T*>(p.bias)[k]) : 0.f;
 #pragma unroll 1
-        for (int h = 0; h < BN / 128; ++h) {        // 128 pixels (two 64-pixel blocks) of the tile at a time
+        for (int h = 0; h < BN / 128; ++h) {        // 128 pixels (128 / PXB blocks) of the tile at a time
           const int ph0 = p0 + h * 128;
-          uint8_t* buf = outbuf + ob * OUT_BUF_BYTES;
+          uint8_t* buf = outbuf + ob * OUTB;
           if (epi_stg) {
             // every thread has copied the previous contents of this buffer out (with two buffers the barrier of the
             // block in between already guarantees that)
@@ -342,16 +409,14 @@ pw_gemm_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant
             uint32_t r[32];
             tmem_ld_32x32(tmem_base + ((uint32_t)(quarter * 32) << 16) + (a * MB + mb) * BN + h * 128 + cc * 32, r);
             tmem_ld_wait();
-            uint8_t* blk = y5 ? buf + (row >> 3) * 2048 + (cc >> 1) * 1024 + (row & 7) * 128
-                                : buf + (cc >> 1) * (128 * 128) + row * 128;
+            constexpr int EPC = 16 / (int)sizeof(T);   // elements per 16-byte chunk
 #pragma unroll
-            for (int q = 0; q < 4; ++q) {
-              uint4 v;
-              v.x = pack_bf16x2(__uint_as_float(r[8 * q + 0]) + bias, __uint_as_float(r[8 * q + 1]) + bias);
-              v.y = pack_bf16x2(__uint_as_float(r[8 * q + 2]) + bias, __uint_as_float(r[8 * q + 3]) + bias);
-              v.z = pack_bf16x2(__uint_as_float(r[8 * q + 4]) + bias, __uint_as_float(r[8 * q + 5]) + bias);
-              v.w = pack_bf16x2(__uint_as_float(r[8 * q + 6]) + bias, __uint_as_float(r[8 * q + 7]) + bias);
-              const int chunk = ((cc & 1) * 4 + q) ^ (row & 7);   // SWIZZLE_128B: 16-B chunk ^ (row % 8)
+            for (int q = 0; q < 32 / EPC; ++q) {
+              const int e = cc * (32 / EPC) + q;       // 16-B chunk of this channel row: block e / 8, chunk e % 8
+              uint8_t* blk = y5 ? buf + (row >> 3) * 2048 + (e >> 3) * 1024 + (row & 7) * 128
+                                  : buf + (e >> 3) * (128 * 128) + row * 128;
+              const uint4 v = Tc<T>::pack16(r + EPC * q, bias);
+              const int chunk = (e & 7) ^ (row & 7);   // SWIZZLE_128B: 16-B chunk ^ (row % 8)
               *reinterpret_cast<uint4*>(blk + chunk * 16) = v;
             }
           }
@@ -374,7 +439,7 @@ pw_gemm_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant
                   const int rw = rr * 16 + r0;
                   if (k0 + rw < p.M) {
                     const uint4 v = *reinterpret_cast<const uint4*>(buf + j * (128 * 128) + rw * 128 + ((g ^ (rw & 7)) << 4));
-                    __stcs(reinterpret_cast<uint4*>(p.y + ((size_t)n * p.M + k0 + rw) * p.P + px), v);
+                    __stcs(reinterpret_cast<uint4*>(static_cast<T*>(p.y) + ((size_t)n * p.M + k0 + rw) * p.P + px), v);
                   }
                 }
               }
@@ -387,12 +452,12 @@ pw_gemm_kernel(const __grid_constant__ CUtensorMap tmap_w, const __grid_constant
                 tma_store_5d(&tmap_y, buf, 0, 0, ph0 >> 6, k0 >> 3, n);
               } else if (ybox == 128) {
 #pragma unroll
-                for (int j = 0; j < 2; ++j) tma_store_3d(&tmap_y, buf + j * (128 * 128), ph0 + j * 64, k0, n);
+                for (int j = 0; j < 128 / PXB; ++j) tma_store_3d(&tmap_y, buf + j * (128 * 128), ph0 + j * PXB, k0, n);
               } else {
                 for (int cg = 0; cg < 128 && k0 + cg < p.M; cg += ybox)
 #pragma unroll
-                  for (int j = 0; j < 2; ++j)
-                    tma_store_3d(&tmap_y, buf + j * (128 * 128) + cg * 128, ph0 + j * 64, k0 + cg, n);
+                  for (int j = 0; j < 128 / PXB; ++j)
+                    tma_store_3d(&tmap_y, buf + j * (128 * 128) + cg * 128, ph0 + j * PXB, k0 + cg, n);
               }
               tma_store_commit();
             }
@@ -442,32 +507,35 @@ inline int sm_count() {
 constexpr int SMEM_LIMIT = 222 * 1024;   // leave room for a small co-resident kernel (halo post/collect, boundary strips)
 constexpr int SMEM_AUX = 1024 /*align*/ + 512 /*barriers*/;
 
-template <int MB, int BN, bool EXT>
+template <typename T, int MB, int BN, bool EXT>
 int launch_pw_ext(const CUtensorMap& tw, const CUtensorMap& tx, const CUtensorMap& tx4, const CUtensorMap& ty, PwParams p,
               cudaStream_t st) {
-  const int kchunks = (p.Cin + BK - 1) / BK;
+  constexpr int OUTB = OUT_BUF_BYTES<T>;
+  const int kchunks = (p.Cin + ROW<T> - 1) / ROW<T>;
   const int budget = SMEM_LIMIT - SMEM_AUX;
   const int wres_bytes = p.taps * kchunks * MB * A_BLK_BYTES;
   const int sms = sm_count();
   int grid = p.num_tiles < sms ? p.num_tiles : sms;
   if (p.num_tiles < 16 * sms) p.tgroup = 1;   // small problems: keep every SM busy
+  // resident filter rows: up to 128 KB with bf16; fp32 (64 KB staging buffer) keeps room for 3 activation stages
+  const int wres_max = sizeof(T) == 2 ? 128 * 1024 : budget - OUTB - 3 * (BN / ROW<T>) * B_BLK_BYTES<T>;
   // stationary weights with several groups of output channels: every CTA serves one group (see the kernel), which needs
   // a grid that is a multiple of num_mg and tiles dealt round-robin
-  bool stationary = wres_bytes <= 128 * 1024;
+  bool stationary = wres_bytes <= wres_max;
   if (stationary && p.num_mg > 1) {
     if (p.stationary_ok && grid >= 4 * p.num_mg) { grid = grid / p.num_mg * p.num_mg; p.tgroup = 1; }
     else stationary = false;
   }
   p.wres = stationary ? 1 : 0;
-  const int stage_bytes = (p.wres ? 0 : MB * A_BLK_BYTES) + (BN / 64) * B_BLK_BYTES;
+  const int stage_bytes = (p.wres ? 0 : MB * A_BLK_BYTES) + (BN / ROW<T>) * B_BLK_BYTES<T>;
   const int rem = budget - (p.wres ? wres_bytes : 0);
   p.out_bufs = 2;
-  p.stages = (rem - 2 * OUT_BUF_BYTES) / stage_bytes;
-  if (p.stages < 3 || env_int("SPC_PW_OUTBUFS", 2) == 1) { p.out_bufs = 1; p.stages = (rem - OUT_BUF_BYTES) / stage_bytes; }
+  p.stages = (rem - 2 * OUTB) / stage_bytes;
+  if (p.stages < 3 || env_int("SPC_PW_OUTBUFS", 2) == 1) { p.out_bufs = 1; p.stages = (rem - OUTB) / stage_bytes; }
   if (p.stages > MAX_STAGES) p.stages = MAX_STAGES;
   SPC_REQUIRE(p.stages >= 2, "tcgen05 conv: shared memory budget too small (MB=%d kchunks=%d)", MB, kchunks);
-  const int smem = (p.wres ? wres_bytes : 0) + p.stages * stage_bytes + p.out_bufs * OUT_BUF_BYTES + SMEM_AUX;
-  auto kern = pw_gemm_kernel<MB, BN, EXT>;
+  const int smem = (p.wres ? wres_bytes : 0) + p.stages * stage_bytes + p.out_bufs * OUTB + SMEM_AUX;
+  auto kern = pw_gemm_kernel<T, MB, BN, EXT>;
   static bool attr_set = false;   // per instantiation
   if (!attr_set) {
     SPC_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
@@ -479,18 +547,26 @@ int launch_pw_ext(const CUtensorMap& tw, const CUtensorMap& tx, const CUtensorMa
   return SPC_OK;
 }
 
-template <int MB, int BN>
+template <typename T, int MB, int BN>
 int launch_pw(const CUtensorMap& tw, const CUtensorMap& tx, const CUtensorMap& tx4, const CUtensorMap& ty, const PwParams& p,
               cudaStream_t st) {
-  const bool ext = p.x5 || p.y5 || p.epi_stg || p.xbox != BK || p.ybox != 128;
-  return ext ? launch_pw_ext<MB, BN, true>(tw, tx, tx4, ty, p, st) : launch_pw_ext<MB, BN, false>(tw, tx, tx4, ty, p, st);
+  if constexpr (sizeof(T) == 4) {   // TF32 launches use none of the round-2 options (run_conv_tc)
+    return launch_pw_ext<T, MB, BN, false>(tw, tx, tx4, ty, p, st);
+  } else {
+    const bool ext = p.x5 || p.y5 || p.epi_stg || p.xbox != ROW<T> || p.ybox != 128;
+    return ext ? launch_pw_ext<T, MB, BN, true>(tw, tx, tx4, ty, p, st)
+               : launch_pw_ext<T, MB, BN, false>(tw, tx, tx4, ty, p, st);
+  }
 }
 
-int make_act_tmap(CUtensorMap* m, const void* base, int P, int Cc, int N, int box_rows) {
+// [N][Cc][P] activations, boxes of one 128-byte row of pixels (64 bf16 / 32 fp32) x box_rows channels
+template <typename T>
+int make_act_tmap(CUtensorMap* m, const void* base, int P, int Cc, int N, int box_rows,
+                  CUtensorMapSwizzle swz = CU_TENSOR_MAP_SWIZZLE_128B) {
   const uint64_t dims[3] = {(uint64_t)P, (uint64_t)Cc, (uint64_t)N};
-  const uint64_t strides[3] = {0, (uint64_t)P * 2, (uint64_t)P * Cc * 2};
-  const uint32_t box[3] = {64, (uint32_t)box_rows, 1};
-  return make_tmap(m, base, 3, dims, strides, box);
+  const uint64_t strides[3] = {0, (uint64_t)P * sizeof(T), (uint64_t)P * Cc * sizeof(T)};
+  const uint32_t box[3] = {(uint32_t)ROW<T>, (uint32_t)box_rows, 1};
+  return make_tmap_sw(m, base, 3, dims, strides, box, swz, Tc<T>::TMA_TYPE);
 }
 
 // [N][Cc][P] bf16 as (64 px, 8 channels, P/64 pixel blocks, Cc/8 channel groups, N): one box = `groups` channel
@@ -502,56 +578,64 @@ int make_act_tmap5(CUtensorMap* m, const void* base, int P, int Cc, int N, int g
   return make_tmap(m, base, 5, dims, strides, box);
 }
 
+template <typename T>
 int launch_shift_copies(const void* x, void* xs, size_t planes, int H, int W, int S, int pw, int cs, cudaStream_t st);
 
 // Geometry of one tcgen05 convolution launch (fprop, or dgrad expressed as a convolution of dY).
+template <typename T>
 struct TcConv {
-  const __nv_bfloat16* w;      // original filter [K][C][R][S]
+  const T* w;                  // original filter [K][C][R][S]
   long long sm, sc;            // strides of (output channel m, reduction channel c) in w
   int flip;                    // rotate taps by 180 degrees (dgrad)
   int M, Cin;                  // output channels, reduction channels
   int R, S, ph, pw;            // filter and zero padding
   int H, W, N;                 // input image
   int stride;                  // 1 or 2 (both axes)
-  const __nv_bfloat16* prepacked;   // if set: weights already in [taps][Mpad][Cpad] layout (1024-aligned)
+  const T* prepacked;          // if set: weights already in [taps][Mpad][Cpad] layout (1024-aligned)
 };
 
 // Y[N][M][H*W] = sum_taps Wp[tap][M x Cin] * shift_tap(X[N][Cin][H][W])  (+bias)
-int run_conv_tc(const TcConv& c, const __nv_bfloat16* x, const __nv_bfloat16* bias, __nv_bfloat16* y, void* ws,
-                size_t ws_bytes, cudaStream_t st) {
+// T = float: TF32 operands; tap convolutions always go through the shifted copies (conv_tap.cu is bf16-only) and none
+// of the bf16 tuning knobs apply.
+template <typename T>
+int run_conv_tc(const TcConv<T>& c, const T* x, const T* bias, T* y, void* ws, size_t ws_bytes, cudaStream_t st) {
+  constexpr bool BF = sizeof(T) == 2;
+  constexpr int BK = ROW<T>;
+  constexpr size_t ES = sizeof(T);
   const int taps = c.R * c.S;
   const int cs = c.stride;
   const int Ho = c.H / cs, Wo = c.W / cs;
   const int Pin = c.H * c.W, P = Ho * Wo;            // P: output pixels per image
   const int Mpad = round_up(c.M, 128), Cpad = round_up(c.Cin, BK);
-  const bool v2 = taps > 1 && !env_get("SPC_TAP_V1") && tap_v2_supported(c.M, c.Cin, c.R, c.S, c.H, c.W, c.N, cs);
+  const bool v2 = BF && taps > 1 && !env_get("SPC_TAP_V1") && tap_v2_supported(c.M, c.Cin, c.R, c.S, c.H, c.W, c.N, cs);
   const bool copies = (c.S > 1 || cs > 1) && taps > 1 && !v2;   // column-shifted (and subsampled) copies of the input
   const uintptr_t ws0 = reinterpret_cast<uintptr_t>(ws);
   const uintptr_t wp_addr = (ws0 + 1023) & ~(uintptr_t)1023;
-  const size_t wp_bytes = c.prepacked ? 0 : (size_t)taps * Mpad * Cpad * 2;
+  const size_t wp_bytes = c.prepacked ? 0 : (size_t)taps * Mpad * Cpad * ES;
   const uintptr_t xs_addr = (wp_addr + wp_bytes + 1023) & ~(uintptr_t)1023;
-  const size_t xs_bytes = copies ? (size_t)c.S * c.N * c.Cin * c.H * Wo * 2 : 0;
+  const size_t xs_bytes = copies ? (size_t)c.S * c.N * c.Cin * c.H * Wo * ES : 0;
   const size_t need = (xs_addr - ws0) + xs_bytes;
   SPC_REQUIRE((ws && ws_bytes >= need) || need <= 1024, "tcgen05 conv: workspace too small (%zu < %zu)", ws_bytes, need);
-  const __nv_bfloat16* wp = c.prepacked;
+  const T* wp = c.prepacked;
   if (!c.prepacked) {
-    __nv_bfloat16* wpm = reinterpret_cast<__nv_bfloat16*>(wp_addr);
+    T* wpm = reinterpret_cast<T*>(wp_addr);
     const int total = taps * Mpad * Cpad;
     int blocks = (total + 255) / 256;
     if (blocks > 1184) blocks = 1184;
-    repack_weights_kernel<<<blocks, 256, 0, st>>>(c.w, wpm, c.M, c.Cin, Mpad, Cpad, taps, c.sm, c.sc, c.flip);
+    repack_weights_kernel<T><<<blocks, 256, 0, st>>>(c.w, wpm, c.M, c.Cin, Mpad, Cpad, taps, c.sm, c.sc, c.flip);
     count_launch();
     SPC_CHECK_CUDA(cudaGetLastError());
     wp = wpm;
   }
-  if (v2)
-    return run_conv_tap_v2(wp, Mpad, Cpad, x, bias, y, c.M, c.Cin, c.R, c.S, c.ph, c.H, c.W, c.N, st);
-  const __nv_bfloat16* xsrc = x;
+  if constexpr (BF) {
+    if (v2) return run_conv_tap_v2(wp, Mpad, Cpad, x, bias, y, c.M, c.Cin, c.R, c.S, c.ph, c.H, c.W, c.N, st);
+  }
+  const T* xsrc = x;
   if (copies) {
     void* xs = reinterpret_cast<void*>(xs_addr);
-    int rc0 = launch_shift_copies(x, xs, (size_t)c.N * c.Cin, c.H, c.W, c.S, c.pw, cs, st);
+    int rc0 = launch_shift_copies<T>(x, xs, (size_t)c.N * c.Cin, c.H, c.W, c.S, c.pw, cs, st);
     if (rc0) return rc0;
-    xsrc = reinterpret_cast<const __nv_bfloat16*>(xs);
+    xsrc = reinterpret_cast<const T*>(xs);
   }
   CUtensorMap tw, tx, tx4, ty;
   // Wide-N variant (256-pixel tiles, one 128-row block of output channels per CTA with its filter rows resident in
@@ -562,41 +646,42 @@ int run_conv_tc(const TcConv& c, const __nv_bfloat16* x, const __nv_bfloat16* bi
   // activation stages fit, and 64 KB in flight per SM at ~2 us of load latency caps the CTA at ~35 GB/s.  Kept behind
   // SPC_PW_N256=1 (off by default); results are bit-identical to the default path.
   const char* n256_env = env_get("SPC_PW_N256");
-  const bool n256 = taps == 1 && cs == 1 && Mpad / 128 >= 3 && (Cpad / BK) * A_BLK_BYTES <= 128 * 1024 && P % 256 == 0 &&
-                    (n256_env ? atoi(n256_env) != 0 : false);
+  const bool n256 = BF && taps == 1 && cs == 1 && Mpad / 128 >= 3 && (Cpad / BK) * A_BLK_BYTES <= 128 * 1024 &&
+                    P % 256 == 0 && (n256_env ? atoi(n256_env) != 0 : false);
   const int BN = n256 ? 256 : BN_DEFAULT;
-  int xbox = (taps == 1) ? env_int("SPC_PW_XBOX", BK) : BK, ybox = env_int("SPC_PW_YBOX", 128);
+  int xbox = (BF && taps == 1) ? env_int("SPC_PW_XBOX", BK) : BK, ybox = BF ? env_int("SPC_PW_YBOX", 128) : 128;
   if (xbox != 8 && xbox != 16 && xbox != 32) xbox = BK;
   if (ybox != 8 && ybox != 16 && ybox != 32 && ybox != 64) ybox = 128;
   // 5-d boxes (see PwParams::x5): measured on B200 (profiles/r2f_pw_box5.txt) +20..32 % on the layers whose channel
   // planes span several 2 MB pages (104->208 @4096^2: 4.30 -> 5.67 TB/s), neutral at 1024^2 planes -> on from 4 MB planes.
-  // SPC_PW_BOX5 = 0..3 overrides (bit 0: activations, bit 1: outputs).
+  // SPC_PW_BOX5 = 0..3 overrides (bit 0: activations, bit 1: outputs).  bf16 only.
   const char* box5_env = env_get("SPC_PW_BOX5");
-  const int box5 = box5_env ? atoi(box5_env) : ((size_t)P * 2 >= ((size_t)4 << 20) ? 3 : 0);
+  const int box5 = !BF ? 0 : box5_env ? atoi(box5_env) : ((size_t)P * 2 >= ((size_t)4 << 20) ? 3 : 0);
   const int x5 = (taps == 1 && cs == 1 && (box5 & 1) && P % 64 == 0 && c.Cin % 8 == 0 && xbox == BK) ? 1 : 0;
   const int y5 = (taps == 1 && (box5 & 2) && P % 64 == 0 && c.M % 8 == 0 && ybox == 128) ? 1 : 0;
   {
     const uint64_t dims[2] = {(uint64_t)Cpad, (uint64_t)taps * Mpad};
-    const uint64_t strides[2] = {0, (uint64_t)Cpad * 2};
-    const uint32_t box[2] = {BK, 128};
-    int rc = make_tmap(&tw, wp, 2, dims, strides, box);
+    const uint64_t strides[2] = {0, (uint64_t)Cpad * ES};
+    const uint32_t box[2] = {(uint32_t)BK, 128};
+    int rc = make_tmap(&tw, wp, 2, dims, strides, box, Tc<T>::TMA_TYPE);
     if (rc) return rc;
   }
   int rc;
   if (taps > 1) {
     // (copies of) the input as [img][Cin][H][Wo]; img = n + s*N for the copy of filter column s
     const uint64_t dims[4] = {(uint64_t)Wo, (uint64_t)c.H, (uint64_t)c.Cin, (uint64_t)c.N * (copies ? c.S : 1)};
-    const uint64_t strides[4] = {0, (uint64_t)Wo * 2, (uint64_t)c.H * Wo * 2, (uint64_t)c.H * Wo * c.Cin * 2};
-    const uint32_t box[4] = {64, 1, BK, 1};
-    rc = make_tmap(&tx4, xsrc, 4, dims, strides, box);
+    const uint64_t strides[4] = {0, (uint64_t)Wo * ES, (uint64_t)c.H * Wo * ES, (uint64_t)c.H * Wo * c.Cin * ES};
+    const uint32_t box[4] = {(uint32_t)ROW<T>, 1, (uint32_t)BK, 1};
+    rc = make_tmap_sw(&tx4, xsrc, 4, dims, strides, box, Tc<T>::B_SWZ, Tc<T>::TMA_TYPE);
     if (rc) return rc;
     tx = tx4;
   } else {
-    rc = x5 ? make_act_tmap5(&tx, x, Pin, c.Cin, c.N, BK / 8, BN / 64) : make_act_tmap(&tx, x, Pin, c.Cin, c.N, xbox);
+    rc = x5 ? make_act_tmap5(&tx, x, Pin, c.Cin, c.N, BK / 8, BN / 64)
+            : make_act_tmap<T>(&tx, x, Pin, c.Cin, c.N, xbox, Tc<T>::B_SWZ);
     if (rc) return rc;
     tx4 = tx;
   }
-  rc = y5 ? make_act_tmap5(&ty, y, P, c.M, c.N, 16, 2) : make_act_tmap(&ty, y, P, c.M, c.N, ybox);
+  rc = y5 ? make_act_tmap5(&ty, y, P, c.M, c.N, 16, 2) : make_act_tmap<T>(&ty, y, P, c.M, c.N, ybox);
   if (rc) return rc;
   PwParams p{};
   p.xbox = xbox; p.ybox = ybox; p.x5 = x5; p.y5 = y5;
@@ -605,7 +690,7 @@ int run_conv_tc(const TcConv& c, const __nv_bfloat16* x, const __nv_bfloat16* bi
   p.shiftN = copies ? c.N : 0;
   p.rowmul = cs;
   p.y = y;
-  p.epi_stg = (env_int("SPC_PW_EPI_STG", 0) == 1 && P % 8 == 0 && !y5) ? 1 : 0;
+  p.epi_stg = (BF && env_int("SPC_PW_EPI_STG", 0) == 1 && P % 8 == 0 && !y5) ? 1 : 0;
   {
     const char* e = env_get("SPC_TILE_GROUP");
     p.tgroup = e ? atoi(e) : 1;   // measured: no effect on B200 (tools/stride_probe.py), kept as a knob
@@ -625,25 +710,34 @@ int run_conv_tc(const TcConv& c, const __nv_bfloat16* x, const __nv_bfloat16* bi
   {
     const char* se = env_get("SPC_PW_STATIONARY");
     const int kch = (c.Cin + BK - 1) / BK;
-    p.stationary_ok = ((se && atoi(se) != 0) || n256) && taps * kch * A_BLK_BYTES <= 128 * 1024;
+    p.stationary_ok = BF && ((se && atoi(se) != 0) || n256) && taps * kch * A_BLK_BYTES <= 128 * 1024;
     if (p.stationary_ok && MBtot >= 3 && !n256) mb = (taps * kch * 2 * A_BLK_BYTES <= 128 * 1024) ? 2 : 1;
     if (n256) mb = 1;
   }
-  if (MBtot >= 3 && !n256 && env_get("SPC_PW_MB4")) mb = 4;                 // A/B knobs
-  if (MBtot >= 3 && !n256 && env_get("SPC_PW_MB2")) mb = 2;
+  if (BF && MBtot >= 3 && !n256 && env_get("SPC_PW_MB4")) mb = 4;                 // A/B knobs
+  if (BF && MBtot >= 3 && !n256 && env_get("SPC_PW_MB2")) mb = 2;
+  // fp32: the 64 KB staging buffer leaves room for at most two 128-row blocks per CTA (3 stages of 48 KB)
+  if (!BF && mb > 2) mb = 2;
   p.num_mg = (MBtot + mb - 1) / mb;
   p.tiles_per_image = (P + BN - 1) / BN;
   p.num_tiles = p.tiles_per_image * c.N * p.num_mg;
-  if (n256) return launch_pw<1, 256>(tw, tx, tx4, ty, p, st);
-  if (mb == 1) return launch_pw<1, 128>(tw, tx, tx4, ty, p, st);
-  if (mb == 2) return launch_pw<2, 128>(tw, tx, tx4, ty, p, st);
-  return launch_pw<4, 128>(tw, tx, tx4, ty, p, st);
+  if constexpr (BF) {
+    if (n256) return launch_pw<T, 1, 256>(tw, tx, tx4, ty, p, st);
+  }
+  if (mb == 1) return launch_pw<T, 1, 128>(tw, tx, tx4, ty, p, st);
+  if constexpr (BF) {
+    if (mb == 2) return launch_pw<T, 2, 128>(tw, tx, tx4, ty, p, st);
+    return launch_pw<T, 4, 128>(tw, tx, tx4, ty, p, st);
+  } else {
+    return launch_pw<T, 2, 128>(tw, tx, tx4, ty, p, st);
+  }
 }
 
 // pointwise helper (1x1): Y[N][M][P] = Wp[M x Cin] * X[N][Cin][P]
-int run_pw(const __nv_bfloat16* w, int ld, int transpose, int M, int Cin, const __nv_bfloat16* x,
-           const __nv_bfloat16* bias, __nv_bfloat16* y, int N, int P, void* ws, size_t ws_bytes, cudaStream_t st) {
-  TcConv c{};
+template <typename T>
+int run_pw(const T* w, int ld, int transpose, int M, int Cin, const T* x, const T* bias, T* y, int N, int P, void* ws,
+           size_t ws_bytes, cudaStream_t st) {
+  TcConv<T> c{};
   c.w = w;
   c.sm = transpose ? 1 : ld; c.sc = transpose ? ld : 1; c.flip = 0;
   c.M = M; c.Cin = Cin; c.R = 1; c.S = 1; c.ph = 0; c.pw = 0; c.H = 1; c.W = P; c.N = N; c.stride = 1;
@@ -677,7 +771,8 @@ struct WgParams {
   int dy5, x5;      // wide stages: operand moves as one 5-d box [8-ch group][px block][8 ch][128 B] (see PwParams::x5)
 };
 
-template <int MG>
+// T = float (TF32 operands): chunks of 32 pixels (one 128-byte row), 3-d boxes only (pb == 1).
+template <typename T, int MG>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 pw_wgrad_kernel(const __grid_constant__ CUtensorMap tmap_dy, const __grid_constant__ CUtensorMap tmap_x,
                 const __grid_constant__ CUtensorMap tmap_x4, const WgParams p) {
@@ -728,7 +823,7 @@ pw_wgrad_kernel(const __grid_constant__ CUtensorMap tmap_dy, const __grid_consta
         WG_DECODE(it)
         (void)mgp;
         for (int ch = c_begin; ch < c_end; ++ch) {
-          const int n = ch / p.chunks_per_image, p0 = (ch % p.chunks_per_image) * (64 * p.pb);
+          const int n = ch / p.chunks_per_image, p0 = (ch % p.chunks_per_image) * (ROW<T> * p.pb);
           mbar_wait(&empty[s], ph ^ 1);
           uint8_t* st = smem + s * stage_bytes;
           mbar_arrive_expect_tx(&full[s], p.pb * (MG * p.mrows * 128 + ntap * b_bytes));
@@ -741,7 +836,7 @@ pw_wgrad_kernel(const __grid_constant__ CUtensorMap tmap_dy, const __grid_consta
                 tma_load_5d(da, &tmap_dy, &full[s], 0, 0, p0 >> 6, r0 >> 3, n);
               } else {
                 tma_load_3d(da, &tmap_dy, &full[s], p0, r0, n);
-                tma_load_3d(da + A_BLK_BYTES, &tmap_dy, &full[s], p0 + 64, r0, n);
+                tma_load_3d(da + A_BLK_BYTES, &tmap_dy, &full[s], p0 + ROW<T>, r0, n);
               }
             }
             uint8_t* xa = st + MG * (2 * A_BLK_BYTES);
@@ -749,7 +844,7 @@ pw_wgrad_kernel(const __grid_constant__ CUtensorMap tmap_dy, const __grid_consta
               tma_load_5d(xa, &tmap_x, &full[s], 0, 0, p0 >> 6, (nb * p.nblk) >> 3, n);
             } else {
               tma_load_3d(xa, &tmap_x, &full[s], p0, nb * p.nblk, n);
-              tma_load_3d(xa + b_slot, &tmap_x, &full[s], p0 + 64, nb * p.nblk, n);
+              tma_load_3d(xa + b_slot, &tmap_x, &full[s], p0 + ROW<T>, nb * p.nblk, n);
             }
             if (++s == p.stages) { s = 0; ph ^= 1; }
             continue;
@@ -773,7 +868,7 @@ pw_wgrad_kernel(const __grid_constant__ CUtensorMap tmap_dy, const __grid_consta
     }
   } else if (warp == 1) {
     if (lane == 0) {
-      const uint32_t idesc = umma_idesc_bf16(128, p.nblk, 0, 0);
+      const uint32_t idesc = Tc<T>::idesc(128, p.nblk, 0, 0);
       int s = 0, ph = 0, aph = 0;
       for (int it = blockIdx.x; it < num_items; it += gridDim.x) {
         WG_DECODE(it)
@@ -798,7 +893,7 @@ pw_wgrad_kernel(const __grid_constant__ CUtensorMap tmap_dy, const __grid_consta
 #pragma unroll
                 for (int i = 0; i < MG; ++i) {
                   const uint64_t adesc = umma_desc(sa + i * (2 * A_BLK_BYTES) + j * aj + ks * 32, 16, asbo);
-                  umma_bf16(tmem_base + i * p.nblk, adesc, bdesc, idesc, (ch > c_begin || ks > 0 || j > 0) ? 1u : 0u);
+                  Tc<T>::mma(tmem_base + i * p.nblk, adesc, bdesc, idesc, (ch > c_begin || ks > 0 || j > 0) ? 1u : 0u);
                 }
               }
             }
@@ -814,7 +909,7 @@ pw_wgrad_kernel(const __grid_constant__ CUtensorMap tmap_dy, const __grid_consta
 #pragma unroll
               for (int i = 0; i < MG; ++i) {
                 const uint64_t adesc = umma_desc(sa + i * A_BLK_BYTES + ks * 32, 16, 1024);
-                umma_bf16(tmem_base + (t * MG + i) * p.nblk, adesc, bdesc, idesc, (ch > c_begin || ks > 0) ? 1u : 0u);
+                Tc<T>::mma(tmem_base + (t * MG + i) * p.nblk, adesc, bdesc, idesc, (ch > c_begin || ks > 0) ? 1u : 0u);
               }
             }
           }
@@ -868,7 +963,7 @@ pw_wgrad_kernel(const __grid_constant__ CUtensorMap tmap_dy, const __grid_consta
   if (warp == 1) tmem_dealloc(tmem_base, TMEM_COLS);
 }
 
-template <int MG>
+template <typename T, int MG>
 int launch_wg(const CUtensorMap& tdy, const CUtensorMap& tx, const CUtensorMap& tx4, WgParams p, cudaStream_t st) {
   const int b_slot = (p.nblk * 128 + 1023) & ~1023;
   // taps per pass: TMEM columns and a stage small enough for >= 2 pipeline stages
@@ -913,7 +1008,7 @@ int launch_wg(const CUtensorMap& tdy, const CUtensorMap& tx, const CUtensorMap& 
   p.splits = splits;
   p.split_major = env_get("SPC_WG_GROUP_MAJOR") ? 0 : 1;            // A/B knob: previous item order
   const int smem = p.stages * stage_bytes + SMEM_AUX;
-  auto kern = pw_wgrad_kernel<MG>;
+  auto kern = pw_wgrad_kernel<T, MG>;
   static bool attr_set = false;
   if (!attr_set) {
     SPC_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_LIMIT));
@@ -1143,8 +1238,12 @@ int launch_wg_pair(const CUtensorMap& tdy, const CUtensorMap& tx, WgParams p, cu
 
 // x: activations [N][C][Hin][Wo] (taps == 1: Hin == Ho) or their S column-shifted (and, for
 // stride 2, column-subsampled) copies [S][N][C][Hin][Wo].  Ho x Wo = extent of dy.
-int run_wgrad(const __nv_bfloat16* x, const __nv_bfloat16* dy, float* dw, int K, int C, int N, int Ho, int Wo, int Hin,
-              int R, int S, int ph, int stride, bool copies, cudaStream_t st) {
+// T = float (TF32 operands): the 1-CTA kernel for every channel count, 32-pixel chunks, 3-d boxes.
+template <typename T>
+int run_wgrad(const T* x, const T* dy, float* dw, int K, int C, int N, int Ho, int Wo, int Hin, int R, int S, int ph,
+              int stride, bool copies, cudaStream_t st) {
+  constexpr bool BF = sizeof(T) == 2;
+  constexpr size_t ES = sizeof(T);
   const int P = Ho * Wo;
   WgParams p{};
   p.dw = dw; p.K = K; p.C = C; p.P = P; p.N = N;
@@ -1160,19 +1259,19 @@ int run_wgrad(const __nv_bfloat16* x, const __nv_bfloat16* dy, float* dw, int K,
   MG = min(MG, env_int("SPC_WG_MG", MG));
   MG = MG >= 4 ? 4 : (MG >= 2 ? 2 : 1);
   p.mgroups = (MBtot + MG - 1) / MG;
-  p.chunks_per_image = (P + 63) / 64;
+  p.chunks_per_image = (P + ROW<T> - 1) / ROW<T>;
   p.chunks_total = p.chunks_per_image * N;
   p.pb = 1;
   // CTA pairs (cta_group::2): measured on B200 (tools/wgrad_probe.py --pair, profiles/r2_wgrad_pair.txt): x1.11..1.32
   // for >= 416 input channels (624->416 @2048^2: 4.95 -> 3.74 ms), break-even at 416->104 / 208->52, slower for
   // the HBM-bound narrow layers (104->208: x0.75, 52->208: x0.67).  SPC_WG_2CTA=1 / SPC_WG_1CTA=1 force either.
-  const bool pair = p.taps == 1 && (env_get("SPC_WG_2CTA") ? true : (env_get("SPC_WG_1CTA") ? false : C >= 400)) &&
+  const bool pair = BF && p.taps == 1 && (env_get("SPC_WG_2CTA") ? true : (env_get("SPC_WG_1CTA") ? false : C >= 400)) &&
                     MBtot >= 2 && p.nblk % 16 == 0;
   // wide stages (two 64-pixel blocks per operand row and stage, 5-d boxes): for 1x1 layers whose channel planes span
   // several 2 MB pages, same reason as PwParams::x5.  SPC_WG_WIDE=0/1 overrides, SPC_WG_BOX5 (bit 0 dy, bit 1 x).
   {
     const char* we = env_get("SPC_WG_WIDE");
-    const bool wide = p.taps == 1 && !pair && P % 128 == 0 && (we ? atoi(we) != 0 : (size_t)P * 2 >= ((size_t)2 << 20));
+    const bool wide = BF && p.taps == 1 && !pair && P % 128 == 0 && (we ? atoi(we) != 0 : (size_t)P * 2 >= ((size_t)2 << 20));
     if (wide) {
       const int b_slot = (p.nblk * 128 + 1023) & ~1023;
       while (MG > 1 && 2 * 2 * (MG * A_BLK_BYTES + b_slot) > SMEM_LIMIT - SMEM_AUX) MG >>= 1;
@@ -1187,17 +1286,17 @@ int run_wgrad(const __nv_bfloat16* x, const __nv_bfloat16* dy, float* dw, int K,
     }
   }
   CUtensorMap tdy, tx, tx4;
-  int rc = p.dy5 ? make_act_tmap5(&tdy, dy, P, K, N, p.mrows / 8, 2) : make_act_tmap(&tdy, dy, P, K, N, p.mrows);
+  int rc = p.dy5 ? make_act_tmap5(&tdy, dy, P, K, N, p.mrows / 8, 2) : make_act_tmap<T>(&tdy, dy, P, K, N, p.mrows);
   if (rc) return rc;
   if (p.taps > 1) {
     const uint64_t dims[4] = {(uint64_t)Wo, (uint64_t)Hin, (uint64_t)C, (uint64_t)N * (copies ? S : 1)};
-    const uint64_t strides[4] = {0, (uint64_t)Wo * 2, (uint64_t)Hin * Wo * 2, (uint64_t)Hin * Wo * C * 2};
-    const uint32_t box[4] = {64, 1, (uint32_t)p.nblk, 1};
-    rc = make_tmap(&tx4, x, 4, dims, strides, box);
+    const uint64_t strides[4] = {0, (uint64_t)Wo * ES, (uint64_t)Hin * Wo * ES, (uint64_t)Hin * Wo * C * ES};
+    const uint32_t box[4] = {(uint32_t)ROW<T>, 1, (uint32_t)p.nblk, 1};
+    rc = make_tmap(&tx4, x, 4, dims, strides, box, Tc<T>::TMA_TYPE);
     if (rc) return rc;
     tx = tx4;
   } else {
-    rc = p.x5 ? make_act_tmap5(&tx, x, P, C, N, p.nblk / 8, 2) : make_act_tmap(&tx, x, P, C, N, p.nblk);
+    rc = p.x5 ? make_act_tmap5(&tx, x, P, C, N, p.nblk / 8, 2) : make_act_tmap<T>(&tx, x, P, C, N, p.nblk);
     if (rc) return rc;
     tx4 = tx;
   }
@@ -1224,15 +1323,15 @@ int run_wgrad(const __nv_bfloat16* x, const __nv_bfloat16* dy, float* dw, int K,
       if (rc) return rc;
       rc = make_act_tmap5(&txh, x, P, C, N, p.nblk / 16, 2);
     } else {
-      rc = make_act_tmap(&txh, x, P, C, N, p.nblk / 2);
+      rc = make_act_tmap<T>(&txh, x, P, C, N, p.nblk / 2);
     }
     if (rc) return rc;
     p.mgroups = (npairs + MP - 1) / MP;
     return MP == 2 ? launch_wg_pair<2>(tdy, txh, p, st) : launch_wg_pair<1>(tdy, txh, p, st);
   }
-  if (MG == 1) return launch_wg<1>(tdy, tx, tx4, p, st);
-  if (MG == 2) return launch_wg<2>(tdy, tx, tx4, p, st);
-  return launch_wg<4>(tdy, tx, tx4, p, st);
+  if (MG == 1) return launch_wg<T, 1>(tdy, tx, tx4, p, st);
+  if (MG == 2) return launch_wg<T, 2>(tdy, tx, tx4, p, st);
+  return launch_wg<T, 4>(tdy, tx, tx4, p, st);
 }
 
 // ---- 3x3 stride-2 dgrad: the four output-parity classes of dX as channel groups of ONE 2x2-tap
@@ -1285,52 +1384,64 @@ __global__ void interleave_s2_kernel(const __nv_bfloat16* __restrict__ t, __nv_b
 }
 
 // ---- stride-2 pointwise convs: subsample / zero-upsample passes around the GEMM ------------------
-// y[n,c,i,j] = x[n,c,2i,2j]; 8 outputs per thread (two 16-byte loads, one 16-byte store)
-__global__ void subsample2_kernel(const __nv_bfloat16* __restrict__ x, __nv_bfloat16* __restrict__ y, size_t planes,
-                                  int H, int W) {
-  const int Ho = H / 2, Wo = W / 2, wv = Wo / 8;
+// y[n,c,i,j] = x[n,c,2i,2j]; one 16-byte output vector per thread (8 bf16 / 4 fp32) from two 16-byte loads
+template <typename T>
+__global__ void subsample2_kernel(const T* __restrict__ x, T* __restrict__ y, size_t planes, int H, int W) {
+  constexpr int V = 16 / (int)sizeof(T);
+  const int Ho = H / 2, Wo = W / 2, wv = Wo / V;
   const size_t total = planes * Ho * wv;
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
     const int v = (int)(i % wv);
     const int oy = (int)((i / wv) % Ho);
     const size_t pl = i / ((size_t)wv * Ho);
-    const uint4* src = reinterpret_cast<const uint4*>(x + (pl * H + 2 * oy) * W + v * 16);
+    const uint4* src = reinterpret_cast<const uint4*>(x + (pl * H + 2 * oy) * W + v * 2 * V);
     const uint4 a = __ldg(src), b = __ldg(src + 1);
     uint4 o;
-    o.x = __byte_perm(a.x, a.y, 0x5410);
-    o.y = __byte_perm(a.z, a.w, 0x5410);
-    o.z = __byte_perm(b.x, b.y, 0x5410);
-    o.w = __byte_perm(b.z, b.w, 0x5410);
-    *reinterpret_cast<uint4*>(y + (pl * Ho + oy) * Wo + v * 8) = o;
+    if constexpr (sizeof(T) == 2) {
+      o.x = __byte_perm(a.x, a.y, 0x5410);
+      o.y = __byte_perm(a.z, a.w, 0x5410);
+      o.z = __byte_perm(b.x, b.y, 0x5410);
+      o.w = __byte_perm(b.z, b.w, 0x5410);
+    } else {
+      o.x = a.x; o.y = a.z; o.z = b.x; o.w = b.z;
+    }
+    *reinterpret_cast<uint4*>(y + (pl * Ho + oy) * Wo + v * V) = o;
   }
 }
 // dx[n,c,2i,2j] = g[n,c,i,j], zero elsewhere
-__global__ void upsample2_zero_kernel(const __nv_bfloat16* __restrict__ g, __nv_bfloat16* __restrict__ dx,
-                                      size_t planes, int H, int W) {
-  const int Ho = H / 2, Wo = W / 2, wv = Wo / 8;
+template <typename T>
+__global__ void upsample2_zero_kernel(const T* __restrict__ g, T* __restrict__ dx, size_t planes, int H, int W) {
+  constexpr int V = 16 / (int)sizeof(T);
+  const int Ho = H / 2, Wo = W / 2, wv = Wo / V;
   const size_t total = planes * Ho * wv;
   const uint4 z = make_uint4(0, 0, 0, 0);
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
     const int v = (int)(i % wv);
     const int oy = (int)((i / wv) % Ho);
     const size_t pl = i / ((size_t)wv * Ho);
-    const uint4 a = __ldg(reinterpret_cast<const uint4*>(g + (pl * Ho + oy) * Wo + v * 8));
+    const uint4 a = __ldg(reinterpret_cast<const uint4*>(g + (pl * Ho + oy) * Wo + v * V));
     uint4 lo, hi;   // element e -> position 2e, zeros between
-    lo.x = a.x & 0xFFFFu; lo.y = a.x >> 16; lo.z = a.y & 0xFFFFu; lo.w = a.y >> 16;
-    hi.x = a.z & 0xFFFFu; hi.y = a.z >> 16; hi.z = a.w & 0xFFFFu; hi.w = a.w >> 16;
-    uint4* d0 = reinterpret_cast<uint4*>(dx + (pl * H + 2 * oy) * W + v * 16);
-    uint4* d1 = reinterpret_cast<uint4*>(dx + (pl * H + 2 * oy + 1) * W + v * 16);
+    if constexpr (sizeof(T) == 2) {
+      lo.x = a.x & 0xFFFFu; lo.y = a.x >> 16; lo.z = a.y & 0xFFFFu; lo.w = a.y >> 16;
+      hi.x = a.z & 0xFFFFu; hi.y = a.z >> 16; hi.z = a.w & 0xFFFFu; hi.w = a.w >> 16;
+    } else {
+      lo.x = a.x; lo.y = 0u; lo.z = a.y; lo.w = 0u;
+      hi.x = a.z; hi.y = 0u; hi.z = a.w; hi.w = 0u;
+    }
+    uint4* d0 = reinterpret_cast<uint4*>(dx + (pl * H + 2 * oy) * W + v * 2 * V);
+    uint4* d1 = reinterpret_cast<uint4*>(dx + (pl * H + 2 * oy + 1) * W + v * 2 * V);
     d0[0] = lo; d0[1] = hi; d1[0] = z; d1[1] = z;
   }
 }
+template <typename T>
 int launch_resample(bool up, const void* src, void* dst, size_t planes, int H, int W, cudaStream_t st) {
-  const size_t total = planes * (H / 2) * (W / 16);
+  const size_t total = planes * (H / 2) * (W / 2 / (16 / sizeof(T)));
   size_t blocks = (total + 255) / 256;
   if (blocks > 148 * 32) blocks = 148 * 32;
   if (up)
-    upsample2_zero_kernel<<<(int)blocks, 256, 0, st>>>((const __nv_bfloat16*)src, (__nv_bfloat16*)dst, planes, H, W);
+    upsample2_zero_kernel<T><<<(int)blocks, 256, 0, st>>>((const T*)src, (T*)dst, planes, H, W);
   else
-    subsample2_kernel<<<(int)blocks, 256, 0, st>>>((const __nv_bfloat16*)src, (__nv_bfloat16*)dst, planes, H, W);
+    subsample2_kernel<T><<<(int)blocks, 256, 0, st>>>((const T*)src, (T*)dst, planes, H, W);
   count_launch();
   SPC_CHECK_CUDA(cudaGetLastError());
   return SPC_OK;
@@ -1342,35 +1453,39 @@ int launch_resample(bool up, const void* src, void* dst, size_t planes, int H, i
 // every tap (r, s) is then an ALIGNED box of copy s at row offset r - ph.
 // With column stride cs (stride-2 convs) the copies are also subsampled:
 //     xs[s][plane][h][j] = x[plane][h][cs*j + s - pw],  j < W/cs.
-__global__ void shift_copies_kernel(const __nv_bfloat16* __restrict__ x, __nv_bfloat16* __restrict__ xs,
-                                    size_t planes, int H, int W, int S, int pw, int cs) {
+// One 16-byte output vector (8 bf16 / 4 fp32) per thread.
+template <typename T>
+__global__ void shift_copies_kernel(const T* __restrict__ x, T* __restrict__ xs, size_t planes, int H, int W, int S,
+                                    int pw, int cs) {
+  constexpr int V = 16 / (int)sizeof(T);
   const int Wv = W / cs;
-  const int wv = Wv / 8;
+  const int wv = Wv / V;
   const size_t rows = planes * H;
   const size_t total = rows * wv * S;
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
     const int v = (int)(i % wv);
     const size_t row = (i / wv) % rows;
     const int sidx = (int)(i / ((size_t)wv * rows));
-    const __nv_bfloat16* src = x + row * W;
-    const int w0 = v * 8 * cs + sidx - pw;
-    __nv_bfloat16 e[8];
+    const T* src = x + row * W;
+    const int w0 = v * V * cs + sidx - pw;
+    T e[V];
 #pragma unroll
-    for (int j = 0; j < 8; ++j) {
+    for (int j = 0; j < V; ++j) {
       const int w = w0 + j * cs;
-      e[j] = ((unsigned)w < (unsigned)W) ? src[w] : __float2bfloat16(0.f);
+      e[j] = ((unsigned)w < (unsigned)W) ? src[w] : Tc<T>::from_float(0.f);
     }
-    *reinterpret_cast<uint4*>(xs + ((size_t)sidx * rows + row) * Wv + v * 8) = *reinterpret_cast<const uint4*>(e);
+    *reinterpret_cast<uint4*>(xs + ((size_t)sidx * rows + row) * Wv + v * V) = *reinterpret_cast<const uint4*>(e);
   }
 }
-// Fast path, stride 1: one thread produces the 8-pixel vector of ALL S copies from three aligned
-// 16-byte loads (previous / own / next vector); a copy shifted by `off` columns is a 16-bit
-// funnel shift of that 24-element window.  |s - pw| <= 8.
-template <int S, int PW>
+// Fast path, stride 1: one thread produces the 16-byte vector (8 bf16 / 4 fp32 pixels) of ALL S copies from three
+// aligned 16-byte loads (previous / own / next vector); a copy shifted by `off` columns is a 16-bit funnel shift
+// (bf16) or a word selection (fp32) of that 3-vector window.  |s - pw| <= 16 B worth of pixels.
+template <typename T, int S, int PW>
 __global__ void __launch_bounds__(256)
-shift_copies_vec_kernel(const __nv_bfloat16* __restrict__ x, __nv_bfloat16* __restrict__ xs, size_t planes, int H,
-                        int W) {
-  const int wv = W / 8;
+shift_copies_vec_kernel(const T* __restrict__ x, T* __restrict__ xs, size_t planes, int H, int W) {
+  constexpr int V = 16 / (int)sizeof(T);
+  static_assert(PW <= V && S - 1 - PW <= V, "shift wider than one vector");
+  const int wv = W / V;
   const size_t rows = planes * H;
   const size_t total = rows * wv;
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
@@ -1384,22 +1499,26 @@ shift_copies_vec_kernel(const __nv_bfloat16* __restrict__ x, __nv_bfloat16* __re
     const uint32_t win[13] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w, c.x, c.y, c.z, c.w, 0u};
 #pragma unroll
     for (int sidx = 0; sidx < S; ++sidx) {
-      const int e0 = 8 + sidx - PW;            // first element of the window [a|b|c]: compile-time
-      const int k = e0 >> 1;
+      const int e0 = V + sidx - PW;            // first element of the window [a|b|c]: compile-time
       uint4 o;
-      if (e0 & 1) {
-        o.x = __funnelshift_r(win[k], win[k + 1], 16);
-        o.y = __funnelshift_r(win[k + 1], win[k + 2], 16);
-        o.z = __funnelshift_r(win[k + 2], win[k + 3], 16);
-        o.w = __funnelshift_r(win[k + 3], win[k + 4], 16);
+      if constexpr (sizeof(T) == 2) {
+        const int k = e0 >> 1;
+        if (e0 & 1) {
+          o.x = __funnelshift_r(win[k], win[k + 1], 16);
+          o.y = __funnelshift_r(win[k + 1], win[k + 2], 16);
+          o.z = __funnelshift_r(win[k + 2], win[k + 3], 16);
+          o.w = __funnelshift_r(win[k + 3], win[k + 4], 16);
+        } else {
+          o.x = win[k]; o.y = win[k + 1]; o.z = win[k + 2]; o.w = win[k + 3];
+        }
       } else {
-        o.x = win[k]; o.y = win[k + 1]; o.z = win[k + 2]; o.w = win[k + 3];
+        o.x = win[e0]; o.y = win[e0 + 1]; o.z = win[e0 + 2]; o.w = win[e0 + 3];
       }
-      *reinterpret_cast<uint4*>(xs + ((size_t)sidx * rows + row) * W + v * 8) = o;
+      *reinterpret_cast<uint4*>(xs + ((size_t)sidx * rows + row) * W + v * V) = o;
     }
   }
 }
-// Fast path, stride 2, 3 filter columns, pw = 1: xs[s][j] = x[2j + s - 1]; 8 outputs per copy from the
+// Fast path, stride 2, 3 filter columns, pw = 1 (bf16): xs[s][j] = x[2j + s - 1]; 8 outputs per copy from the
 // own 16 input pixels plus the last pixel of the previous vector.
 __global__ void __launch_bounds__(256)
 shift_copies_s2k3_kernel(const __nv_bfloat16* __restrict__ x, __nv_bfloat16* __restrict__ xs, size_t planes, int H,
@@ -1428,24 +1547,26 @@ shift_copies_s2k3_kernel(const __nv_bfloat16* __restrict__ x, __nv_bfloat16* __r
     *reinterpret_cast<uint4*>(dst + 2 * rows * Wv) = od;                  // s = 2: 2j + 1
   }
 }
+template <typename T>
 int launch_shift_copies(const void* x, void* xs, size_t planes, int H, int W, int S, int pw, int cs, cudaStream_t st) {
+  constexpr int V = 16 / (int)sizeof(T);
   const bool aligned = (reinterpret_cast<uintptr_t>(x) % 16 == 0) && (reinterpret_cast<uintptr_t>(xs) % 16 == 0);
-  if (aligned && cs == 1 && W % 8 == 0 &&
+  if (aligned && cs == 1 && W % V == 0 &&
       ((S == 7 && pw == 3) || (S == 3 && pw == 1) || (S == 5 && pw == 2) || (S == 2 && pw == 0))) {
-    const size_t tot = planes * H * (W / 8);
+    const size_t tot = planes * H * (W / V);
     size_t blocks = (tot + 255) / 256;
     if (blocks > 148 * 32) blocks = 148 * 32;
-    const __nv_bfloat16* xi = (const __nv_bfloat16*)x;
-    __nv_bfloat16* xo = (__nv_bfloat16*)xs;
-    if (S == 7) shift_copies_vec_kernel<7, 3><<<(int)blocks, 256, 0, st>>>(xi, xo, planes, H, W);
-    else if (S == 3) shift_copies_vec_kernel<3, 1><<<(int)blocks, 256, 0, st>>>(xi, xo, planes, H, W);
-    else if (S == 5) shift_copies_vec_kernel<5, 2><<<(int)blocks, 256, 0, st>>>(xi, xo, planes, H, W);
-    else shift_copies_vec_kernel<2, 0><<<(int)blocks, 256, 0, st>>>(xi, xo, planes, H, W);
+    const T* xi = (const T*)x;
+    T* xo = (T*)xs;
+    if (S == 7) shift_copies_vec_kernel<T, 7, 3><<<(int)blocks, 256, 0, st>>>(xi, xo, planes, H, W);
+    else if (S == 3) shift_copies_vec_kernel<T, 3, 1><<<(int)blocks, 256, 0, st>>>(xi, xo, planes, H, W);
+    else if (S == 5) shift_copies_vec_kernel<T, 5, 2><<<(int)blocks, 256, 0, st>>>(xi, xo, planes, H, W);
+    else shift_copies_vec_kernel<T, 2, 0><<<(int)blocks, 256, 0, st>>>(xi, xo, planes, H, W);
     count_launch();
     SPC_CHECK_CUDA(cudaGetLastError());
     return SPC_OK;
   }
-  if (aligned && cs == 2 && S == 3 && pw == 1 && W % 16 == 0) {
+  if (sizeof(T) == 2 && aligned && cs == 2 && S == 3 && pw == 1 && W % 16 == 0) {
     const size_t tot = planes * H * (W / 16);
     size_t blocks = (tot + 255) / 256;
     if (blocks > 148 * 32) blocks = 148 * 32;
@@ -1454,10 +1575,10 @@ int launch_shift_copies(const void* x, void* xs, size_t planes, int H, int W, in
     SPC_CHECK_CUDA(cudaGetLastError());
     return SPC_OK;
   }
-  const size_t total = planes * H * (W / cs / 8) * S;
+  const size_t total = planes * H * (W / cs / V) * S;
   size_t blocks = (total + 255) / 256;
   if (blocks > 148 * 32) blocks = 148 * 32;
-  shift_copies_kernel<<<(int)blocks, 256, 0, st>>>((const __nv_bfloat16*)x, (__nv_bfloat16*)xs, planes, H, W, S, pw, cs);
+  shift_copies_kernel<T><<<(int)blocks, 256, 0, st>>>((const T*)x, (T*)xs, planes, H, W, S, pw, cs);
   count_launch();
   SPC_CHECK_CUDA(cudaGetLastError());
   return SPC_OK;
@@ -1465,21 +1586,27 @@ int launch_shift_copies(const void* x, void* xs, size_t planes, int H, int W, in
 
 inline bool is_s2(const spc_conv_desc* d) { return d->stride_h == 2 && d->stride_w == 2; }
 inline size_t align1k(size_t b) { return (b + 1023) & ~(size_t)1023; }
+// fp32 storage runs on the tensor cores only when asked for TF32 (SPC_ALGO_TF32); its default is the exact direct kernel
+inline bool is_tf32(const spc_conv_desc* d) { return d->dtype == SPC_F32 && d->algo == SPC_ALGO_TF32; }
+inline size_t elem_bytes(const spc_conv_desc* d) { return d->dtype == SPC_BF16 ? 2 : 4; }
+inline int row_elems(const spc_conv_desc* d) { return 128 / (int)elem_bytes(d); }   // channels per stage (BK)
 
-bool tap_shape_ok(const spc_conv_desc* d) {   // odd RxS "same" convs, stride 1 or 2, on 64-pixel output row segments
-  if (d->dtype != SPC_BF16) return false;
+// odd RxS "same" convs, stride 1 or 2 (TF32: stride 1 only), on 64-pixel output row segments
+bool tap_shape_ok(const spc_conv_desc* d) {
+  if (d->dtype != SPC_BF16 && !is_tf32(d)) return false;
   if (d->R * d->S == 1 || d->R * d->S > 49) return false;
   if ((d->R & 1) == 0 || (d->S & 1) == 0) return false;
   const bool s1 = d->stride_h == 1 && d->stride_w == 1, s2 = d->stride_h == 2 && d->stride_w == 2;
   if (!s1 && !s2) return false;
   if (s2 && (d->H % 2 || d->W % 2)) return false;
+  if (s2 && is_tf32(d)) return false;   // 3x3 stride 2 in fp32 stays on the direct kernel
   const int Wo = d->W / d->stride_w;
   if (Wo % 64 != 0) return false;
   return (long long)d->H * d->W < (1ll << 31);
 }
 
 bool pw_shape_ok(const spc_conv_desc* d) {
-  if (d->dtype != SPC_BF16) return false;
+  if (d->dtype != SPC_BF16 && !is_tf32(d)) return false;
   if (d->R != 1 || d->S != 1) return false;
   long long P = (long long)d->H * d->W;
   if (is_s2(d)) {
@@ -1488,7 +1615,8 @@ bool pw_shape_ok(const spc_conv_desc* d) {
   } else if (d->stride_h != 1 || d->stride_w != 1) {
     return false;
   }
-  if (P % 8 != 0 || P >= (1ll << 31)) return false;
+  // TMA strides are multiples of 16 bytes: P % 8 (bf16) / P % 4 (fp32)
+  if (P % (16 / (long long)elem_bytes(d)) != 0 || P >= (1ll << 31)) return false;
   return true;
 }
 
@@ -1506,17 +1634,19 @@ bool tc_supported(const spc_conv_desc* d, int op) {
 
 // workspace = [repacked weights | subsampled activations (stride-2 only)]
 static size_t wbytes(const spc_conv_desc* d, int op) {
-  const size_t taps = (size_t)d->R * d->S;
-  if (op == 0) return align1k(taps * round_up(d->K, 128) * round_up(d->C, BK) * 2 + 1024);
-  if (op == 1) return align1k(taps * round_up(d->C, 128) * round_up(d->K, BK) * 2 + 1024);
+  const size_t taps = (size_t)d->R * d->S, es = elem_bytes(d);
+  const int bk = row_elems(d);
+  if (op == 0) return align1k(taps * round_up(d->K, 128) * round_up(d->C, bk) * es + 1024);
+  if (op == 1) return align1k(taps * round_up(d->C, 128) * round_up(d->K, bk) * es + 1024);
   return 0;
 }
 size_t tc_workspace_bytes(const spc_conv_desc* d, int op) {
-  const size_t taps = (size_t)d->R * d->S;
+  const size_t taps = (size_t)d->R * d->S, es = elem_bytes(d);
   const int cs = d->stride_w;
+  const bool bf = d->dtype == SPC_BF16;
   size_t b = wbytes(d, op) + 4096;
   if (taps == 1) {
-    if (is_s2(d)) b += align1k((size_t)d->N * d->C * (d->H / 2) * (d->W / 2) * 2) + 1024;
+    if (is_s2(d)) b += align1k((size_t)d->N * d->C * (d->H / 2) * (d->W / 2) * es) + 1024;
     return b;
   }
   const size_t Ho = d->H / cs, Wo = d->W / cs;
@@ -1526,45 +1656,103 @@ size_t tc_workspace_bytes(const spc_conv_desc* d, int op) {
     b += align1k(2ull * d->N * d->K * Ho * Wo * 2) + align1k(4ull * d->N * d->C * Ho * Wo * 2) + 4096;
     return b;
   }
-  if (op != 2 && !env_get("SPC_TAP_V1") &&
+  if (bf && op != 2 && !env_get("SPC_TAP_V1") &&
       tap_v2_supported(op == 1 ? d->C : d->K, op == 1 ? d->K : d->C, d->R, d->S, d->H, d->W, d->N, cs))
     return b;               // conv_tap.cu forms the horizontal taps in shared memory: no copies
-  if (op == 2 && !env_get("SPC_TAP_V1") && wgrad_tap_supported(d->K, d->C, d->R, d->S, d->H, d->W, cs))
+  if (bf && op == 2 && !env_get("SPC_TAP_V1") && wgrad_tap_supported(d->K, d->C, d->R, d->S, d->H, d->W, cs))
     return b;               // wgrad_tap.cu likewise
   if (d->S > 1 || cs > 1)   // S column-shifted (stride 2: also subsampled) copies of the conv input
-    b += align1k((size_t)d->S * d->N * (op == 1 ? d->K : d->C) * d->H * Wo * 2) + 2048;
+    b += align1k((size_t)d->S * d->N * (op == 1 ? d->K : d->C) * d->H * Wo * es) + 2048;
   return b;
 }
+
+namespace {
+
+template <typename T>
+int conv_fwd_t(const spc_conv_desc* d, const T* x, const T* w, const T* bias, T* y, void* ws, size_t ws_bytes,
+               cudaStream_t st) {
+  if (d->R * d->S > 1) {
+    TcConv<T> c{};
+    c.w = w;
+    c.sm = (long long)d->C * d->R * d->S; c.sc = (long long)d->R * d->S; c.flip = 0;
+    c.M = d->K; c.Cin = d->C; c.R = d->R; c.S = d->S; c.ph = d->pad_h; c.pw = d->pad_w;
+    c.H = d->H; c.W = d->W; c.N = d->N; c.stride = d->stride_h;
+    return run_conv_tc(c, x, bias, y, ws, ws_bytes, st);
+  }
+  if (is_s2(d)) {   // Y = W * subsample(X)
+    T* xs = reinterpret_cast<T*>(align1k(reinterpret_cast<uintptr_t>(ws) + wbytes(d, 0)));
+    int rc = launch_resample<T>(false, x, xs, (size_t)d->N * d->C, d->H, d->W, st);
+    if (rc) return rc;
+    return run_pw(w, d->C, 0, d->K, d->C, xs, bias, y, d->N, (d->H / 2) * (d->W / 2), ws, wbytes(d, 0), st);
+  }
+  return run_pw(w, d->C, 0, d->K, d->C, x, bias, y, d->N, d->H * d->W, ws, ws_bytes, st);
+}
+
+// every dgrad except 3x3 stride 2 (bf16 only, tc_conv_dgrad)
+template <typename T>
+int conv_dgrad_t(const spc_conv_desc* d, const T* dy, const T* w, T* dx, void* ws, size_t ws_bytes, cudaStream_t st) {
+  if (d->R * d->S > 1) {   // stride-1 dgrad = correlation of dY with the transposed, 180-degree rotated filter
+    TcConv<T> c{};
+    c.w = w;
+    c.sm = (long long)d->R * d->S; c.sc = (long long)d->C * d->R * d->S; c.flip = 1;
+    c.M = d->C; c.Cin = d->K; c.R = d->R; c.S = d->S; c.ph = d->R - 1 - d->pad_h; c.pw = d->S - 1 - d->pad_w;
+    c.H = d->H; c.W = d->W; c.N = d->N; c.stride = 1;
+    return run_conv_tc(c, dy, (const T*)nullptr, dx, ws, ws_bytes, st);
+  }
+  if (is_s2(d)) {   // dX = zero_upsample(W^T * dY)
+    T* gs = reinterpret_cast<T*>(align1k(reinterpret_cast<uintptr_t>(ws) + wbytes(d, 1)));
+    int rc = run_pw(w, d->C, 1, d->C, d->K, dy, (const T*)nullptr, gs, d->N, (d->H / 2) * (d->W / 2), ws, wbytes(d, 1), st);
+    if (rc) return rc;
+    return launch_resample<T>(true, gs, dx, (size_t)d->N * d->C, d->H, d->W, st);
+  }
+  return run_pw(w, d->C, 1, d->C, d->K, dy, (const T*)nullptr, dx, d->N, d->H * d->W, ws, ws_bytes, st);
+}
+
+template <typename T>
+int conv_wgrad_t(const spc_conv_desc* d, const T* x, const T* dy, float* dw, void* ws, size_t ws_bytes,
+                 cudaStream_t st) {
+  if (d->R * d->S > 1) {
+    const int cs = d->stride_h;
+    if constexpr (sizeof(T) == 2) {
+      if (!env_get("SPC_TAP_V1") && wgrad_tap_supported(d->K, d->C, d->R, d->S, d->H, d->W, cs))
+        return run_wgrad_tap(x, dy, dw, d->K, d->C, d->N, d->H, d->W, d->R, d->S, st);
+    }
+    const bool copies = d->S > 1 || cs > 1;
+    if (copies) {
+      SPC_REQUIRE(ws && ws_bytes >= tc_workspace_bytes(d, 2), "tcgen05 wgrad: workspace too small");
+      void* xs = reinterpret_cast<void*>(align1k(reinterpret_cast<uintptr_t>(ws)));
+      int rc = launch_shift_copies<T>(x, xs, (size_t)d->N * d->C, d->H, d->W, d->S, d->pad_w, cs, st);
+      if (rc) return rc;
+      x = reinterpret_cast<const T*>(xs);
+    }
+    return run_wgrad(x, dy, dw, d->K, d->C, d->N, d->H / cs, d->W / cs, d->H, d->R, d->S, d->pad_h, cs, copies, st);
+  }
+  if (is_s2(d)) {
+    SPC_REQUIRE(ws && ws_bytes >= tc_workspace_bytes(d, 2), "tcgen05 wgrad: workspace too small");
+    T* xs = reinterpret_cast<T*>(align1k(reinterpret_cast<uintptr_t>(ws)));
+    int rc = launch_resample<T>(false, x, xs, (size_t)d->N * d->C, d->H, d->W, st);
+    if (rc) return rc;
+    return run_wgrad<T>(xs, dy, dw, d->K, d->C, d->N, 1, (d->H / 2) * (d->W / 2), 1, 1, 1, 0, 1, false, st);
+  }
+  return run_wgrad(x, dy, dw, d->K, d->C, d->N, 1, d->H * d->W, 1, 1, 1, 0, 1, false, st);
+}
+
+}  // namespace
 
 int tc_conv_fwd(const spc_conv_desc* d, const void* x, const void* w, const void* bias, void* y, void* ws,
                 size_t ws_bytes, cudaStream_t st) {
   SPC_REQUIRE(ws && ws_bytes >= tc_workspace_bytes(d, 0), "tcgen05 conv: workspace too small");
-  if (d->R * d->S > 1) {
-    TcConv c{};
-    c.w = reinterpret_cast<const __nv_bfloat16*>(w);
-    c.sm = (long long)d->C * d->R * d->S; c.sc = (long long)d->R * d->S; c.flip = 0;
-    c.M = d->K; c.Cin = d->C; c.R = d->R; c.S = d->S; c.ph = d->pad_h; c.pw = d->pad_w;
-    c.H = d->H; c.W = d->W; c.N = d->N; c.stride = d->stride_h;
-    return run_conv_tc(c, reinterpret_cast<const __nv_bfloat16*>(x), reinterpret_cast<const __nv_bfloat16*>(bias),
-                       reinterpret_cast<__nv_bfloat16*>(y), ws, ws_bytes, st);
-  }
-  if (is_s2(d)) {   // Y = W * subsample(X)
-    void* xs = reinterpret_cast<void*>(align1k(reinterpret_cast<uintptr_t>(ws) + wbytes(d, 0)));
-    int rc = launch_resample(false, x, xs, (size_t)d->N * d->C, d->H, d->W, st);
-    if (rc) return rc;
-    return run_pw(reinterpret_cast<const __nv_bfloat16*>(w), d->C, 0, d->K, d->C,
-                  reinterpret_cast<const __nv_bfloat16*>(xs), reinterpret_cast<const __nv_bfloat16*>(bias),
-                  reinterpret_cast<__nv_bfloat16*>(y), d->N, (d->H / 2) * (d->W / 2), ws, wbytes(d, 0), st);
-  }
-  return run_pw(reinterpret_cast<const __nv_bfloat16*>(w), d->C, 0, d->K, d->C,
-                reinterpret_cast<const __nv_bfloat16*>(x), reinterpret_cast<const __nv_bfloat16*>(bias),
-                reinterpret_cast<__nv_bfloat16*>(y), d->N, d->H * d->W, ws, ws_bytes, st);
+  if (d->dtype == SPC_F32)
+    return conv_fwd_t(d, (const float*)x, (const float*)w, (const float*)bias, (float*)y, ws, ws_bytes, st);
+  return conv_fwd_t(d, (const __nv_bfloat16*)x, (const __nv_bfloat16*)w, (const __nv_bfloat16*)bias,
+                    (__nv_bfloat16*)y, ws, ws_bytes, st);
 }
 
 int tc_conv_dgrad(const spc_conv_desc* d, const void* dy, const void* w, void* dx, void* ws, size_t ws_bytes,
                   cudaStream_t st) {
   // dX[C x P] = W^T[C x K] * dY[K x P]
   SPC_REQUIRE(ws && ws_bytes >= tc_workspace_bytes(d, 1), "tcgen05 conv: workspace too small");
+  if (d->dtype == SPC_F32) return conv_dgrad_t(d, (const float*)dy, (const float*)w, (float*)dx, ws, ws_bytes, st);
   if (d->R * d->S > 1 && is_s2(d)) {   // 3x3 stride 2: four parity classes as channel groups, then interleave
     const int Ho = d->H / 2, Wo = d->W / 2;
     const int Mq = 4 * d->C, Mpad = round_up(Mq, 128), Kpad = round_up(d->K, BK);
@@ -1581,10 +1769,10 @@ int tc_conv_dgrad(const spc_conv_desc* d, const void* dy, const void* w, void* d
       count_launch();
       SPC_CHECK_CUDA(cudaGetLastError());
     }
-    TcConv c{};
+    TcConv<__nv_bfloat16> c{};
     c.prepacked = wq;
     c.M = Mq; c.Cin = d->K; c.R = 2; c.S = 2; c.ph = 0; c.pw = 0; c.H = Ho; c.W = Wo; c.N = d->N; c.stride = 1;
-    int rc = run_conv_tc(c, reinterpret_cast<const __nv_bfloat16*>(dy), nullptr, tmp, reinterpret_cast<void*>(a),
+    int rc = run_conv_tc(c, reinterpret_cast<const __nv_bfloat16*>(dy), (const __nv_bfloat16*)nullptr, tmp, reinterpret_cast<void*>(a),
                          ws_bytes - (a - reinterpret_cast<uintptr_t>(ws)), st);
     if (rc) return rc;
     const size_t total = (size_t)d->N * d->C * 2 * Ho * (Wo / 8);
@@ -1595,57 +1783,15 @@ int tc_conv_dgrad(const spc_conv_desc* d, const void* dy, const void* w, void* d
     SPC_CHECK_CUDA(cudaGetLastError());
     return SPC_OK;
   }
-  if (d->R * d->S > 1) {   // stride-1 dgrad = correlation of dY with the transposed, 180-degree rotated filter
-    TcConv c{};
-    c.w = reinterpret_cast<const __nv_bfloat16*>(w);
-    c.sm = (long long)d->R * d->S; c.sc = (long long)d->C * d->R * d->S; c.flip = 1;
-    c.M = d->C; c.Cin = d->K; c.R = d->R; c.S = d->S; c.ph = d->R - 1 - d->pad_h; c.pw = d->S - 1 - d->pad_w;
-    c.H = d->H; c.W = d->W; c.N = d->N; c.stride = 1;
-    return run_conv_tc(c, reinterpret_cast<const __nv_bfloat16*>(dy), nullptr, reinterpret_cast<__nv_bfloat16*>(dx), ws,
-                       ws_bytes, st);
-  }
-  if (is_s2(d)) {   // dX = zero_upsample(W^T * dY)
-    void* gs = reinterpret_cast<void*>(align1k(reinterpret_cast<uintptr_t>(ws) + wbytes(d, 1)));
-    int rc = run_pw(reinterpret_cast<const __nv_bfloat16*>(w), d->C, 1, d->C, d->K,
-                    reinterpret_cast<const __nv_bfloat16*>(dy), nullptr, reinterpret_cast<__nv_bfloat16*>(gs), d->N,
-                    (d->H / 2) * (d->W / 2), ws, wbytes(d, 1), st);
-    if (rc) return rc;
-    return launch_resample(true, gs, dx, (size_t)d->N * d->C, d->H, d->W, st);
-  }
-  return run_pw(reinterpret_cast<const __nv_bfloat16*>(w), d->C, 1, d->C, d->K,
-                reinterpret_cast<const __nv_bfloat16*>(dy), nullptr, reinterpret_cast<__nv_bfloat16*>(dx), d->N,
-                d->H * d->W, ws, ws_bytes, st);
+  return conv_dgrad_t(d, (const __nv_bfloat16*)dy, (const __nv_bfloat16*)w, (__nv_bfloat16*)dx, ws, ws_bytes, st);
 }
 
 int tc_conv_wgrad(const spc_conv_desc* d, const void* x, const void* dy, float* dw, int accumulate, void* ws,
                   size_t ws_bytes, cudaStream_t st) {
   // the kernel accumulates with atomics; api.cu has already zeroed dw when !accumulate
   (void)accumulate;
-  const __nv_bfloat16* xb = reinterpret_cast<const __nv_bfloat16*>(x);
-  const __nv_bfloat16* dyb = reinterpret_cast<const __nv_bfloat16*>(dy);
-  if (d->R * d->S > 1) {
-    const int cs = d->stride_h;
-    if (!env_get("SPC_TAP_V1") && wgrad_tap_supported(d->K, d->C, d->R, d->S, d->H, d->W, cs))
-      return run_wgrad_tap(xb, dyb, dw, d->K, d->C, d->N, d->H, d->W, d->R, d->S, st);
-    const bool copies = d->S > 1 || cs > 1;
-    if (copies) {
-      SPC_REQUIRE(ws && ws_bytes >= tc_workspace_bytes(d, 2), "tcgen05 wgrad: workspace too small");
-      void* xs = reinterpret_cast<void*>(align1k(reinterpret_cast<uintptr_t>(ws)));
-      int rc = launch_shift_copies(x, xs, (size_t)d->N * d->C, d->H, d->W, d->S, d->pad_w, cs, st);
-      if (rc) return rc;
-      xb = reinterpret_cast<const __nv_bfloat16*>(xs);
-    }
-    return run_wgrad(xb, dyb, dw, d->K, d->C, d->N, d->H / cs, d->W / cs, d->H, d->R, d->S, d->pad_h, cs, copies, st);
-  }
-  if (is_s2(d)) {
-    SPC_REQUIRE(ws && ws_bytes >= tc_workspace_bytes(d, 2), "tcgen05 wgrad: workspace too small");
-    void* xs = reinterpret_cast<void*>(align1k(reinterpret_cast<uintptr_t>(ws)));
-    int rc = launch_resample(false, x, xs, (size_t)d->N * d->C, d->H, d->W, st);
-    if (rc) return rc;
-    return run_wgrad(reinterpret_cast<const __nv_bfloat16*>(xs), dyb, dw, d->K, d->C, d->N, 1, (d->H / 2) * (d->W / 2), 1,
-                     1, 1, 0, 1, false, st);
-  }
-  return run_wgrad(xb, dyb, dw, d->K, d->C, d->N, 1, d->H * d->W, 1, 1, 1, 0, 1, false, st);
+  if (d->dtype == SPC_F32) return conv_wgrad_t(d, (const float*)x, (const float*)dy, dw, ws, ws_bytes, st);
+  return conv_wgrad_t(d, (const __nv_bfloat16*)x, (const __nv_bfloat16*)dy, dw, ws, ws_bytes, st);
 }
 
 // Y[M][P] = W[M][Cin] * X[Cin][P] (bf16; w row-major with leading dimension ld) and dW[K][C] += dY[K][P] * X[C][P]^T on

@@ -134,6 +134,16 @@ __device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t a_desc, uint
       ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
+// D[tmem] (+)= A[smem desc] * B[smem desc], fp32 storage read as TF32 operands (K = 8 per MMA), fp32 accumulate.
+__device__ __forceinline__ void umma_tf32(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc,
+                                          uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
+      ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
+      : "memory");
+}
 // mbarrier arrives when all tcgen05 ops issued so far by this thread have completed
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar))
@@ -224,19 +234,28 @@ __device__ __forceinline__ void umma_commit_2sm(uint64_t* bar) {
 }
 
 // ---- UMMA shared-memory descriptors (cute/arch/mma_sm100_desc.hpp SmemDescriptor) -----------------
-//  [0,14) start>>4 | [16,30) LBO>>4 | [32,46) SBO>>4 | [46,48) version=1 | [61,64) layout (2 = SWIZZLE_128B)
-__device__ __forceinline__ uint64_t umma_desc(uint32_t smem_addr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
+//  [0,14) start>>4 | [16,30) LBO>>4 | [32,46) SBO>>4 | [46,48) version=1 | [61,64) layout
+//  layout 2 = SWIZZLE_128B (16-byte chunks permuted, TMA CU_TENSOR_MAP_SWIZZLE_128B); layout 1 = SWIZZLE_128B with
+//  32-byte atoms (TMA CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B), the form an MN-major TF32 operand takes
+constexpr uint32_t UMMA_SW128 = 2, UMMA_SW128_ATOM32 = 1;
+__device__ __forceinline__ uint64_t umma_desc(uint32_t smem_addr, uint32_t lbo_bytes, uint32_t sbo_bytes,
+                                              uint32_t layout = UMMA_SW128) {
   uint64_t d = 0;
   d |= (uint64_t)((smem_addr & 0x3FFFF) >> 4);
   d |= (uint64_t)((lbo_bytes >> 4) & 0x3FFF) << 16;
   d |= (uint64_t)((sbo_bytes >> 4) & 0x3FFF) << 32;
   d |= 1ull << 46;
-  d |= 2ull << 61;
+  d |= (uint64_t)layout << 61;
   return d;
 }
 // Instruction descriptor (InstrDescriptor): fp32 accum, bf16 A/B.
 __host__ __device__ constexpr uint32_t umma_idesc_bf16(int M, int N, int a_mn_major, int b_mn_major) {
   return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)a_mn_major << 15) | ((uint32_t)b_mn_major << 16) |
+         ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
+}
+// Same with TF32 A/B (format code 2 of kind::tf32 in bits [7,10) and [10,13)).
+__host__ __device__ constexpr uint32_t umma_idesc_tf32(int M, int N, int a_mn_major, int b_mn_major) {
+  return (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)a_mn_major << 15) | ((uint32_t)b_mn_major << 16) |
          ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
 

@@ -17,6 +17,7 @@ libspconv.so loads.
 """
 import ctypes as C
 import math
+import os
 
 import torch
 import torch.distributed as dist
@@ -31,6 +32,40 @@ _DIRS = [(-1, -1), (-1, 0), (-1, 1), (0, -1), (0, 0), (0, 1), (1, -1), (1, 0), (
 
 def _stream():
     return C.c_void_p(torch.cuda.current_stream().cuda_stream)
+
+
+# Math of fp32 convolutions: "ieee" (default) runs them in exact fp32 on the direct kernels, "tf32" lets the tensor
+# cores read their operands as TF32 (10-bit mantissa, fp32 accumulate and output).  The initial value comes from the
+# SPCONV_FP32_MATH environment variable.  bf16 convolutions and modules with an explicit `algo` are not affected.
+_FP32_MATH_MODES = ("ieee", "tf32")
+
+
+def _parse_fp32_math(mode, source):
+    if mode not in _FP32_MATH_MODES:
+        raise ValueError("%s: fp32 math must be one of %s, got %r" % (source, ", ".join(_FP32_MATH_MODES), mode))
+    return mode
+
+
+_fp32_math = _parse_fp32_math(os.environ.get("SPCONV_FP32_MATH", "ieee"), "SPCONV_FP32_MATH")
+
+
+def set_fp32_math(mode):
+    """Select the math of fp32 conv_spatial / local_conv2d layers: "ieee" (exact fp32, the default) or "tf32"
+    (tensor cores with TF32 operands)."""
+    global _fp32_math
+    _fp32_math = _parse_fp32_math(mode, "set_fp32_math")
+
+
+def get_fp32_math():
+    return _fp32_math
+
+
+def _algo_for(algo, dtype):
+    """Descriptor algo of a module whose `algo` attribute is `algo`: AUTO becomes TF32 for fp32 tensors when the
+    fp32 math is "tf32"; an explicitly chosen algo is passed through."""
+    if algo == _lib.SPC_ALGO_AUTO and dtype == torch.float32 and _fp32_math == "tf32":
+        return _lib.SPC_ALGO_TF32
+    return algo
 
 
 def _require_cuda(t, who):
@@ -328,7 +363,7 @@ class conv_spatial(nn.Conv2d, _SpatialTopology):
             x, et, el = self._fused_pre(x)
         N, Cc, H, W = x.shape
         desc_args = (N, Cc, H, W, self.out_channels, self.kernel_size[0], self.kernel_size[1], self.stride[0],
-                     self.stride[1], hh, hw, _lib.dtype_code(x.dtype), self.algo)
+                     self.stride[1], hh, hw, _lib.dtype_code(x.dtype), _algo_for(self.algo, x.dtype))
         exchange = (hh > 0 or hw > 0) and not self.fused_halo and self.neighbours is not None and any(self.neighbours)
         extra = ()
         with torch.no_grad():
@@ -506,7 +541,7 @@ class local_conv2d(nn.Conv2d):
         N, Cc, H, W = x.shape
         ph, pw = self._same
         desc_args = (N, Cc, H, W, self.out_channels, self.kernel_size[0], self.kernel_size[1], self.stride[0],
-                     self.stride[1], ph, pw, _lib.dtype_code(x.dtype), self.algo)
+                     self.stride[1], ph, pw, _lib.dtype_code(x.dtype), _algo_for(self.algo, x.dtype))
         y = _ConvSpatialFn.apply(x, self.weight, self.bias, desc_args, *([None] * 9))
         ch, cw = ph - self.padding[0], pw - self.padding[1]
         if ch or cw:
